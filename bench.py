@@ -421,6 +421,8 @@ def run_grid(a):
     launches = int(L.bmm_launch_count() - l0)
     clk = clocks.stop()
     plan.check()      # a chain that stopped with an error status invalidates the timing
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, plan.fetch())
     plan.close()
 
     # e2e: the public call with host buffers (bit-packed rows in, uint8 allocation history out)
@@ -537,6 +539,31 @@ def run_grid(a):
     if dist:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_LIMIT = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, res):
+    """--dump-outputs: the arrays a caller of the timed path receives from its last step, one DIR/<name>.npy each, in the
+    returned layout (float64 as computed, integer arrays as float32, which holds labels exactly).  When together they
+    exceed 64 MB, every array keeps the same fraction of its elements, taken at seeded positions that depend only on
+    the array's name and shape: element i of the file is element idx[i] of the row-major flattened array, idx sorted.
+    Two builds run with the same arguments therefore write files that compare element for element."""
+    import zlib
+    os.makedirs(dirname, exist_ok=True)
+    res = {k: np.asarray(v) for k, v in res.items()}
+    size = lambda v: v.size * (8 if v.dtype == np.float64 else 4)
+    total = sum(size(v) for v in res.values())
+    frac = min(1.0, (DUMP_LIMIT - 4096 * len(res)) / max(total, 1))       # 4 KB per file for the .npy header
+    for name, v in sorted(res.items()):
+        if frac < 1.0:
+            m = max(1, int(v.size * frac))
+            idx = np.sort(np.random.default_rng([zlib.crc32(name.encode()), *v.shape]).choice(v.size, m, replace=False))
+            v = v[np.unravel_index(idx, v.shape)]
+        np.save(os.path.join(dirname, name + ".npy"), v.astype(np.float64 if v.dtype == np.float64 else np.float32))
+    print("bench: wrote %d arrays to %s (%s of every array)" % (len(res), dirname, "all" if frac == 1.0 else "%.3g" % frac),
+          file=sys.stderr)
 
 
 def _max_over_ranks(x, dist):
@@ -700,7 +727,12 @@ def main():
     ap.add_argument("--nsamples", type=int, default=None)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip extra.sharded / extra.collapsed_1024 on the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (rank 0; sampled to 64 MB "
+                         "after fetching the whole list into host memory, 15 GB at the C2 size)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm only times the CPU oracle")
     if a.workload in GRID_WORKLOADS:
         if a.impl == "reference":
             return run_grid_reference(a)
@@ -754,6 +786,18 @@ def main():
         if dist:
             dist.barrier()
 
+    # The e2e arm, and --dump-outputs before it, receive the reference's list layout: S x N int32 allocation matrices,
+    # 15 GB per rank at the C2 size -- never drive the box out of memory for it; checked before anything is allocated
+    need = (2 if relabel else 1) * C_ * S * N * 4 * int(os.environ.get("LOCAL_WORLD_SIZE", world))
+    try:
+        import psutil
+        avail = psutil.virtual_memory().available
+    except Exception:
+        avail = None
+    if avail is not None and need > 0.8 * avail:
+        raise SystemExit("bench: the e2e leg needs %.0f GB of host memory for the returned histories, %.0f GB available"
+                         % (need / 1e9, avail / 1e9))
+
     # ---- device-resident arm (value) --------------------------------------------------------
     plan = api.Plan(sid, X, ns, K, chains=C_, seed=2026, device=local, chain_offset=rank * C_, **init_kw, **kw)
     clocks = ClockSampler(local)
@@ -774,20 +818,11 @@ def main():
     launches = int(L.bmm_launch_count() - l0)
     clk = clocks.stop()
     plan.check()      # a chain that stopped with an error status invalidates the timing
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, plan.fetch())
     plan.close()
 
     # ---- end-to-end arm (e2e): the public call with host buffers, every step ------------------
-    # (the reference's list layout: S x N int32 allocation matrices, 15 GB per rank at the C2 size -- never drive the box
-    #  out of memory for it)
-    need = (2 if relabel else 1) * C_ * S * N * 4 * int(os.environ.get("LOCAL_WORLD_SIZE", world))
-    try:
-        import psutil
-        avail = psutil.virtual_memory().available
-    except Exception:
-        avail = None
-    if avail is not None and need > 0.8 * avail:
-        raise SystemExit("bench: the e2e leg needs %.0f GB of host memory for the returned histories, %.0f GB available"
-                         % (need / 1e9, avail / 1e9))
     bufs = api._alloc_out(sid, C_, N, P, K, ns, burnin, relabel, False, (), True)  # pinned
     host_out = api.out_nbytes(bufs[0])
     # bytes that actually cross PCIe: int32 z matrices above 8M allocations travel as 1 B per allocation and

@@ -65,12 +65,18 @@ def has_ref():
     return bool(lib().oracle_has_lpsolve_ref())
 
 
-def assign(cost, use_ref=True):
+def _use_ref(use_ref):
+    """use_ref=None: the reference's lp_solve when oracle/_ref is built, else the exact Hungarian solver.  Both return
+    the unique optimum of a cost matrix without ties; only True insists on lp_solve (and its tie-break)."""
+    return int(has_ref() if use_ref is None else bool(use_ref))
+
+
+def assign(cost, use_ref=None):
     """my_lpsolve: K x K cost -> K x K 0/1 solution."""
     cost = np.asfortranarray(cost, dtype=np.float64)
     K = cost.shape[0]
     sol = np.zeros((K, K), dtype=np.int32, order="F")
-    rc = lib().oracle_assign(K, _dp(cost), _ip(sol), int(use_ref))
+    rc = lib().oracle_assign(K, _dp(cost), _ip(sol), _use_ref(use_ref))
     if rc:
         raise RuntimeError("oracle_assign rc=%d" % rc)
     return sol
@@ -89,25 +95,25 @@ def set_sample_stable(on):
     lib().oracle_set_sample_stable(int(bool(on)))
 
 
-def stephens_batch(p, use_ref=True):
+def stephens_batch(p, use_ref=None):
     p = np.asfortranarray(p, dtype=np.float64)
     N, K, M = p.shape
     q = np.zeros((N, K), order="F")
     perm = np.zeros((M, K), dtype=np.int32, order="F")
-    rc = lib().oracle_stephens_batch(N, K, M, _dp(p), _dp(q), int(use_ref), _ip(perm))
+    rc = lib().oracle_stephens_batch(N, K, M, _dp(p), _dp(q), _use_ref(use_ref), _ip(perm))
     if rc:
         raise RuntimeError("oracle_stephens_batch rc=%d" % rc)
     return q, perm
 
 
-def stephens_online(q, p, sample_num, use_ref=True):
+def stephens_online(q, p, sample_num, use_ref=None):
     q = np.asfortranarray(q, dtype=np.float64)
     p = np.asfortranarray(p, dtype=np.float64)
     N, K = p.shape
     perm = np.zeros(K, dtype=np.int32)
     qn = np.zeros((N, K), order="F")
     cost = np.zeros((K, K), order="F")
-    rc = lib().oracle_stephens_online(N, K, _dp(q), _dp(p), int(sample_num), _ip(perm), _dp(qn), int(use_ref), _dp(cost))
+    rc = lib().oracle_stephens_online(N, K, _dp(q), _dp(p), int(sample_num), _ip(perm), _dp(qn), _use_ref(use_ref), _dp(cost))
     if rc:
         raise RuntimeError("oracle_stephens_online rc=%d" % rc)
     return perm, qn, cost
@@ -216,7 +222,7 @@ def _df(X):
 
 
 def gibbs_full(X, initial_pi, initial_theta, nsamples, K, alpha=0.0, beta=0.5, gamma=0.5, a=1.0, b=1.0,
-               burnin=None, relabel=False, burnrelabel=50, seed=1, use_ref=True, probes=True, stabilise=False,
+               burnin=None, relabel=False, burnrelabel=50, seed=1, use_ref=None, probes=True, stabilise=False,
                stickbreaking=False):
     X = _df(X)
     N, P = X.shape
@@ -227,7 +233,7 @@ def gibbs_full(X, initial_pi, initial_theta, nsamples, K, alpha=0.0, beta=0.5, g
     ith = np.asfortranarray(initial_theta, dtype=np.float64)
     fn = lib().oracle_gibbs_stickbreaking if stickbreaking else lib().oracle_gibbs_full
     rc = fn(_ip(X), N, P, _dp(ipi), _dp(ith), nsamples, K, C.c_double(alpha), C.c_double(beta), C.c_double(gamma),
-            C.c_double(a), C.c_double(b), burnin, int(relabel), burnrelabel, C.c_uint(seed), int(use_ref),
+            C.c_double(a), C.c_double(b), burnin, int(relabel), burnrelabel, C.c_uint(seed), _use_ref(use_ref),
             int(stabilise), C.byref(o))
     if rc:
         raise RuntimeError("oracle sampler rc=%d" % rc)
@@ -240,7 +246,7 @@ def gibbs_stickbreaking(X, initial_pi, initial_theta, nsamples, maxK, **kw):
 
 
 def gibbs_collapsed(X, initial_K, nsamples, K, alpha=0.0, beta=0.5, gamma=0.5, a=1.0, b=1.0, burnin=None,
-                    relabel=False, burnrelabel=50, seed=1, use_ref=True, probes=True):
+                    relabel=False, burnrelabel=50, seed=1, use_ref=None, probes=True):
     X = _df(X)
     N, P = X.shape
     if burnin is None:
@@ -249,7 +255,7 @@ def gibbs_collapsed(X, initial_K, nsamples, K, alpha=0.0, beta=0.5, gamma=0.5, a
     iz = np.asarray(initial_K, dtype=np.int32)
     rc = lib().oracle_gibbs_collapsed(_ip(X), N, P, _ip(iz), nsamples, K, C.c_double(alpha), C.c_double(beta),
                                       C.c_double(gamma), C.c_double(a), C.c_double(b), burnin, int(relabel),
-                                      burnrelabel, C.c_uint(seed), int(use_ref), C.byref(o))
+                                      burnrelabel, C.c_uint(seed), _use_ref(use_ref), C.byref(o))
     if rc:
         raise RuntimeError("oracle sampler rc=%d" % rc)
     r.update(nsamples=nsamples, burnin=burnin, relabel=relabel)
@@ -257,7 +263,7 @@ def gibbs_collapsed(X, initial_K, nsamples, K, alpha=0.0, beta=0.5, gamma=0.5, a
 
 
 def gibbs_dp(X, nsamples, alpha=0.0, beta=0.5, gamma=0.5, a=1.0, b=1.0, burnin=None, relabel=False,
-             burnrelabel=50, maxK=30, seed=1, use_ref=True, probes=True):
+             burnrelabel=50, maxK=30, seed=1, use_ref=None, probes=True):
     X = _df(X)
     N, P = X.shape
     if burnin is None:
@@ -267,7 +273,7 @@ def gibbs_dp(X, nsamples, alpha=0.0, beta=0.5, gamma=0.5, a=1.0, b=1.0, burnin=N
     o.Kactive = _ip(r["Kactive"])
     rc = lib().oracle_gibbs_dp(_ip(X), N, P, nsamples, C.c_double(alpha), C.c_double(beta), C.c_double(gamma),
                                C.c_double(a), C.c_double(b), burnin, int(relabel), burnrelabel, maxK,
-                               C.c_uint(seed), int(use_ref), C.byref(o))
+                               C.c_uint(seed), _use_ref(use_ref), C.byref(o))
     if rc:
         raise RuntimeError("oracle sampler rc=%d" % rc)
     r.update(nsamples=nsamples, burnin=burnin, relabel=relabel)
