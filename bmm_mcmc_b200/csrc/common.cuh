@@ -27,11 +27,14 @@ __host__ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
     return c;
 }
 
-// 53-bit uniform in (0,1) from two 32-bit words
+// 53-bit uniform in (0,1) from two 32-bit words.  (2^53 - 0.5) / 2^53 rounds to 1.0, so the top value is clamped to
+// the largest double below 1: an inverse-CDF draw at u = 1 would run past every category with mass.
 __host__ __device__ __forceinline__ double u53(uint32_t a, uint32_t b) {
     uint64_t v = ((uint64_t)a << 21) ^ (uint64_t)(b >> 11);
-    return ((double)v + 0.5) * (1.0 / 9007199254740992.0);
+    return fmin(((double)v + 0.5) * (1.0 / 9007199254740992.0), 0x1.fffffffffffffp-1);
 }
+// A u53 uniform cast to float: every u53 >= 1 - 2^-25 rounds to 1.0f, so it is clamped to the largest float below 1.
+__host__ __device__ __forceinline__ float unit_f(double u) { return fminf((float)u, 0x1.fffffep-1f); }
 
 // Allocation draws of the uncollapsed samplers: observation gi of sweep j uses word gi & 3 of
 // Philox(counter = (gi >> 2, gi >> 34, stream, j)), i.e. one Philox evaluation serves four consecutive
@@ -41,7 +44,11 @@ __host__ __device__ __forceinline__ uint32_t philox_word(const uint4 &r, int h) 
     return h == 0 ? r.x : (h == 1 ? r.y : (h == 2 ? r.z : r.w));
 }
 __host__ __device__ __forceinline__ double u32_unit(uint32_t w) { return ((double)w + 0.5) * (1.0 / 4294967296.0); }
-__host__ __device__ __forceinline__ float u32_unit_f(uint32_t w) { return ((float)(w >> 8) + 0.5f) * 5.9604644775390625e-08f; }
+// 24-bit float uniform: 16777215.5 rounds to 2^24 in float, so every w >= 0xFFFFFF00 would give exactly 1.0f; those are
+// clamped to the largest float below 1 (all other words keep their value).
+__host__ __device__ __forceinline__ float u32_unit_f(uint32_t w) {
+    return fminf(((float)(w >> 8) + 0.5f) * 5.9604644775390625e-08f, 0x1.fffffep-1f);
+}
 
 // Sequential stream for the (rare, rejection-based) parameter draws.
 // key = (seed_lo, chain); counter = (attempt, index, stream, sweep ^ seed_hi-mix)

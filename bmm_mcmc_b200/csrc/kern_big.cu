@@ -125,6 +125,10 @@ __global__ void __launch_bounds__(BIG_THREADS) big_sweep_kernel(const BigParams 
                 c2 += exp_r<R>(lpi[k] + row_loglik<R>(xb, P, K, k, w1, w0) - mx) / cum;
                 if (u < (double)c2) { z = k; break; }
             }
+            // In float the prefix sum of the first K - 1 probabilities can fall a few ulp short of a u near 1: the draw
+            // then lands on K - 1 whatever its weight.  Fall back to the last cluster with weight instead.
+            if (sizeof(R) == 4 && z == K - 1)
+                while (z > 0 && !(exp_r<R>(lpi[z] + row_loglik<R>(xb, P, K, z, w1, w0) - mx) > (R)0)) --z;
         }
         if (p.probs_f32) {
             for (int k = 0; k < K; ++k)

@@ -220,6 +220,9 @@ __global__ void __launch_bounds__(LP_THREADS, 1) lp_sweep_kernel(const BigParams
             }
             tc_fence_before();
             mbar_arrive(accempty);             // the accumulators may be overwritten by the next super-tile
+            // This walk adds the same values in the same order as the total, so at the last cluster with weight run == sum
+            // > target = u * sum for every u < 1 (u32_unit_f stays below 1): clusters of weight 0 after it are never
+            // counted, and the clamp only guards against a NaN total.
             z = min(z, K - 1);
             if (valid) zrow[i] = (uint8_t)(z + 1);
         };

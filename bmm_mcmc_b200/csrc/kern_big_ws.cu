@@ -393,7 +393,17 @@ __global__ void __launch_bounds__(WS_THREADS, 1) big_sweep_ws_kernel(const BigPa
                 }
                 over += __popc(mask);
             }
-            const int z = min(WS_KC - over, K - 1);
+            int z = min(WS_KC - over, K - 1);
+            // (target - off_g) - c_q can round to >= 0 for the last cluster with weight, and then also for the clusters of
+            // weight 0 after it (a pi_k = 0, or an underflowed 2^l), which would be counted too.  That takes a target within
+            // a few ulp of the total, i.e. u > 1 - 2^-16 (one row in 65 536, so the check stays off the common path): the
+            // draw then falls back to the last cluster with weight, found from where the group prefix sums grow.
+            if (u > 0x1.fffep-1f) {
+                int last = 0;
+#pragma unroll
+                for (int q = 0; q < WS_KC; ++q) last = l[q] > ((q & 7) ? l[q - 1] : 0.f) ? q : last;
+                z = min(z, last);
+            }
             if (valid && zrow) zrow[i] = (uint8_t)(z + 1);
             if (blockIdx.x == 0 && tid == 256) { if (k == 0) ws_stamp(2); if (k + WS_NEPI >= T) ws_stamp(3); }
             if (k >= WS_NB) ok = mbar_wait(b2_free + 8 * b, ph_b ^ 1u);

@@ -445,7 +445,7 @@ __global__ void __launch_bounds__(32) collapsed_prod_kernel(const CollapsedParam
             const int src = (i & 63) >> 1;
             const uint32_t w0 = __shfl_sync(0xffffffffu, (i & 1) ? rnd.z : rnd.x, src);
             const uint32_t w1 = __shfl_sync(0xffffffffu, (i & 1) ? rnd.w : rnd.y, src);
-            const R u = (R)u53(w0, w1);
+            const R u = sizeof(R) == 4 ? (R)unit_f(u53(w0, w1)) : (R)u53(w0, w1);
             const int own = (lane == a);
             const int Nk1 = Nk - own;
             const R ownr = own ? (R)1 : (R)0;
@@ -475,6 +475,8 @@ __global__ void __launch_bounds__(32) collapsed_prod_kernel(const CollapsedParam
                 tot = cum[WIDTH - 1];
                 const R target = u * tot;
                 z = 0;
+                // tot is the last of these serial prefix sums, so every cum from the last cluster with weight on equals tot
+                // > u * tot (u < 1, also as a float): an empty cluster after it is never counted
 #pragma unroll
                 for (int k = 0; k < WIDTH - 1; ++k) z += (k < K - 1 && !(target < cum[k])) ? 1 : 0;
             } else {
@@ -488,8 +490,12 @@ __global__ void __launch_bounds__(32) collapsed_prod_kernel(const CollapsedParam
                     const R t = shfl_r<R>(cum, lane >= off ? lane - off : lane);
                     if (lane >= off) cum += t;
                 }
-                const unsigned hit = __ballot_sync(0xffffffffu, lane < K - 1 && target < cum);
-                z = hit ? __ffs(hit) - 1 : K - 1;
+                // The total is a butterfly sum and cum a scan: they round differently, so target can pass every cum, and
+                // a scan entry of an empty cluster can exceed its predecessor's.  Only clusters with weight are drawn;
+                // when no prefix passes the target the draw falls back to the last cluster with weight.
+                const unsigned hit = __ballot_sync(0xffffffffu, lane < K - 1 && v > (R)0 && target < cum);
+                const unsigned live = __ballot_sync(0xffffffffu, v > (R)0);
+                z = hit ? __ffs(hit) - 1 : (live ? 31 - __clz(live) : K - 1);
             }
             if (!(tot > (R)0) || !isfinite(tot)) { if (lane == 0) p.status[c] = -9; }
             if (need_probs && lane < K) {
