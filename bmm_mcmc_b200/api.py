@@ -17,7 +17,7 @@ import numpy as np
 from . import _lib
 from .rcompat import RRng
 
-__all__ = ["gibbs_full", "gibbs_collapsed", "gibbs_dp", "gibbs_stickbreaking", "Plan", "PackedX"]
+__all__ = ["gibbs_full", "gibbs_collapsed", "gibbs_dp", "gibbs_stickbreaking", "predictive", "waic", "Plan", "PackedX"]
 
 
 def _r_round(x):
@@ -416,4 +416,62 @@ def predictive(fit, newdata, membership=True):
     out = {"log_pred": lp}
     if membership:
         out["membership"] = np.ascontiguousarray(mem.T)
+    return out
+
+
+def _waic_draws(fit):
+    """theta [C][K x P x S] and pi [C][S x K] in the C ABI's memory order, from a fit with or without a chain axis."""
+    if "pi" not in fit:
+        raise ValueError("waic() needs the pi history of an uncollapsed sampler (gibbs_full / gibbs_stickbreaking)")
+    th, pi = np.asarray(fit["theta"], dtype=np.float64), np.asarray(fit["pi"], dtype=np.float64)
+    chains = th.ndim == 4
+    if not chains:
+        th, pi = th[None], pi[None]
+    if th.ndim != 4 or pi.ndim != 3:
+        raise ValueError("theta must be K x P x S (C x K x P x S) and pi S x K (C x S x K)")
+    Cn, K, P, S = th.shape
+    if pi.shape != (Cn, S, K):
+        raise ValueError("theta / pi shapes do not match")
+    return (np.ascontiguousarray(th.transpose(0, 3, 2, 1)), np.ascontiguousarray(pi.transpose(0, 2, 1)),
+            Cn, K, P, S, chains)
+
+
+def waic(fit, data, *, no_tensor=False, device=0):
+    """WAIC of a fitted `gibbs_full` / `gibbs_stickbreaking` model and the log-likelihood trace of its draws, computed on the
+    device (Watanabe 2010; Vehtari, Gelman & Gabry 2017, the layout of R's `loo::waic`).
+
+    `data` is the N x P 0/1 matrix the model was fitted to, or a `PackedX`.  With a chain axis the C chains' S draws are
+    pooled (D = C S >= 2).  With l[c,s,i] = log p(x_i | draw (c, s)): `pointwise_lppd` = log mean exp l, `pointwise_p_waic`
+    = the sample variance of l over the draws, `pointwise_elpd_waic` = their difference, `pointwise_waic` = -2 times it;
+    the totals are sums over i and `se_*` = sqrt(N var_i(pointwise)).  `loglik[c, s]` = sum_i l[c,s,i], the trace.  With a
+    chain axis `chain_elpd_waic`, `chain_waic` and `chain_p_waic` are the same totals from each chain's draws alone.
+
+    K <= 32 and P <= 112 fits with many distinct rows run on the tcgen05 kernel (fp16 hi|lo operands, fp32 log-sum-exp,
+    fp64 moments); `no_tensor=True` forces the fp64 kernel."""
+    th, pi, Cn, K, P, S, chains = _waic_draws(fit)
+    X = _as_X(data)
+    N = X.shape[0]
+    if X.shape[1] != P:
+        raise ValueError("data has %d columns, theta has %d variables" % (X.shape[1], P))
+    if Cn * S < 2:
+        raise ValueError("waic needs at least 2 draws")
+    flags = (_lib.FLAG_X_PACKED if isinstance(X, PackedX) else 0) | (_lib.FLAG_NO_TENSOR if no_tensor else 0)
+    ll = np.zeros((Cn, S))
+    lppd, pw = np.zeros(N), np.zeros(N)
+    clp, cpw = np.zeros(Cn), np.zeros(Cn)
+    xp = X.bits.ctypes.data if isinstance(X, PackedX) else X.ctypes.data
+    _lib.check(_lib.lib().bmm_waic(C.c_void_p(xp), N, P, K, S, Cn, _p(th, C.c_double), _p(pi, C.c_double), flags,
+                                   int(device), _p(ll, C.c_double), _p(lppd, C.c_double), _p(pw, C.c_double),
+                                   _p(clp, C.c_double), _p(cpw, C.c_double)))
+    elpd = lppd - pw
+    out = {"pointwise_lppd": lppd, "pointwise_p_waic": pw, "pointwise_elpd_waic": elpd, "pointwise_waic": -2.0 * elpd}
+    for name in ("lppd", "p_waic", "elpd_waic", "waic"):
+        v = out["pointwise_" + name]
+        out[name] = float(v.sum())
+        out["se_" + name] = float(np.sqrt(N * np.var(v, ddof=1))) if N > 1 else float("nan")
+    out["loglik"] = ll if chains else ll[0]
+    if chains:
+        out["chain_elpd_waic"] = clp - cpw
+        out["chain_waic"] = -2.0 * (clp - cpw)
+        out["chain_p_waic"] = cpw
     return out

@@ -121,14 +121,6 @@ struct DevBuf {
     template <typename T> T *as() const { return (T *)p; }
 };
 
-struct VecHash {
-    size_t operator()(const std::vector<uint32_t> &v) const {
-        uint64_t h = 1469598103934665603ull;
-        for (uint32_t w : v) { h ^= w; h *= 1099511628211ull; }
-        return (size_t)h;
-    }
-};
-
 }  // namespace
 
 struct bmm_plan {
@@ -271,6 +263,36 @@ int upload(DevBuf &b, const T *src, size_t n) {
 
 #define TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
 
+// De-duplicate bit-packed rows [N][W] in first-occurrence order: rowid[i] = index of row i among the U distinct rows,
+// wt[u] = multiplicity of distinct row u, rowbits = the distinct rows [U][W].  The hash set keys on row indices and
+// reads the words in place, so N = 1e7 rows need no per-row allocation.
+void dedup_rows(const uint32_t *bits, int N, int W, std::vector<int> &rowid, std::vector<int> &wt,
+                std::vector<uint32_t> &rowbits) {
+    auto hash = [&](int i) {
+        uint64_t h = 1469598103934665603ull;
+        for (int w = 0; w < W; ++w) { h ^= bits[(size_t)i * W + w]; h *= 1099511628211ull; }
+        return (size_t)h;
+    };
+    auto eq = [&](int i, int j) { return std::memcmp(bits + (size_t)i * W, bits + (size_t)j * W, (size_t)W * 4) == 0; };
+    std::unordered_map<int, int, decltype(hash), decltype(eq)> seen(std::min(N, 1 << 20), hash, eq);
+    rowid.assign(N, 0);
+    wt.clear();
+    rowbits.clear();
+    for (int i = 0; i < N; ++i) {
+        auto it = seen.find(i);
+        if (it == seen.end()) {
+            const int u = (int)wt.size();
+            seen.emplace(i, u);
+            wt.push_back(1);
+            rowbits.insert(rowbits.end(), bits + (size_t)i * W, bits + (size_t)(i + 1) * W);
+            rowid[i] = u;
+        } else {
+            wt[it->second]++;
+            rowid[i] = it->second;
+        }
+    }
+}
+
 int create_full(bmm_plan *pl, const bmm_init *init) {
     const bmm_args &a = pl->a;
     const int N = pl->N, P = pl->P, K = pl->K, C = pl->C, ns = pl->ns, S = pl->S;
@@ -278,27 +300,9 @@ int create_full(bmm_plan *pl, const bmm_init *init) {
     int W;
     TRY(pack_rows(a.X, N, P, bits, W));
     pl->W = W;
-    // de-duplicate rows (first-occurrence order)
-    std::vector<int> rowid(N), wt;
+    std::vector<int> rowid, wt;
     std::vector<uint32_t> rowbits;
-    {
-        std::unordered_map<std::vector<uint32_t>, int, VecHash> seen;
-        std::vector<uint32_t> key(W);
-        for (int i = 0; i < N; ++i) {
-            for (int w = 0; w < W; ++w) key[w] = bits[(size_t)i * W + w];
-            auto it = seen.find(key);
-            if (it == seen.end()) {
-                int u = (int)wt.size();
-                seen.emplace(key, u);
-                wt.push_back(1);
-                rowbits.insert(rowbits.end(), key.begin(), key.end());
-                rowid[i] = u;
-            } else {
-                wt[it->second]++;
-                rowid[i] = it->second;
-            }
-        }
-    }
+    dedup_rows(bits.data(), N, W, rowid, wt, rowbits);
     const int U = (int)wt.size();
     pl->U = U;
     const size_t UK = (size_t)U * K, KP = (size_t)K * P;
@@ -1502,6 +1506,121 @@ int bmm_predictive(const int32_t *Xnew, int32_t M, int32_t P, int32_t K, int32_t
                            membership ? mem.as<double>() : nullptr, 0));
     CU(cudaMemcpy(log_pred, lp.p, (size_t)M * 8, cudaMemcpyDeviceToHost));
     if (membership) CU(cudaMemcpy(membership, mem.p, (size_t)M * K * 8, cudaMemcpyDeviceToHost));
+    return BMM_OK;
+}
+
+// WAIC and the log-likelihood trace of C chains x S kept draws (kern_predict.cu, kern_waic_tc.cu).  The rows are
+// de-duplicated first; the tcgen05 kernel takes shapes it covers once there are enough distinct rows to give every SM
+// tiles of its own (below that the fp64 kernel's split of the draws over warps is the faster, DESIGN.md section 4).
+static thread_local float g_waic_ms = 0.f;
+static thread_local int32_t g_waic_tensor = 0;
+static constexpr int WAIC_TC_MIN_TILES_PER_SM = 1;
+
+int bmm_waic(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta, const double *pi,
+             uint32_t flags, int32_t device, double *loglik, double *lppd, double *p_waic, double *chain_lppd,
+             double *chain_p_waic) {
+    if (!X || !theta || !pi || N < 1 || P < 1 || K < 1 || K > 255 || S < 1 || C < 1)
+        return fail(BMM_ERR_INVALID, "bad waic arguments");
+    const long long D = (long long)C * S;
+    if (D < 2) return fail(BMM_ERR_INVALID, "waic needs at least 2 draws (C * S >= 2)");
+    if (D > 0x7FFFFFFFLL) return fail(BMM_ERR_INVALID, "waic: C * S too large");
+    if (device < 0 || bmm_device_count() <= device) return fail(BMM_ERR_CUDA, "no CUDA device (this library has no CPU fallback)");
+    std::vector<uint32_t> bits;
+    int W = (P + 31) / 32;
+    if (flags & BMM_FLAG_X_PACKED) {
+        const uint32_t *xb = (const uint32_t *)X, tail = (P & 31) ? (1u << (P & 31)) - 1u : ~0u;
+        bits.assign(xb, xb + (size_t)N * W);
+        for (int i = 0; i < N; ++i) bits[(size_t)i * W + W - 1] &= tail;   // bits beyond P are not part of the row
+    } else {
+        TRY(pack_rows((const int32_t *)X, N, P, bits, W));
+    }
+    std::vector<int> rowid, wt;
+    std::vector<uint32_t> rowbits;
+    dedup_rows(bits.data(), N, W, rowid, wt, rowbits);
+    std::vector<uint32_t>().swap(bits);
+    const int U = (int)wt.size();
+    // pi [C][S x K cm] -> D x K cm over the chain-major draws g = c S + s (theta [C][K x P x S] already is K x P x D)
+    std::vector<double> pid((size_t)D * K);
+    for (int c = 0; c < C; ++c)
+        for (int k = 0; k < K; ++k)
+            for (int s = 0; s < S; ++s) pid[(size_t)c * S + s + (size_t)D * k] = pi[(size_t)c * S * K + s + (size_t)S * k];
+    CU(cudaSetDevice(device));
+    int sms = 0;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    const int ntc = (U + 127) / 128;
+    const char *force = getenv("BMM_WAIC_TENSOR");   // tests: the tcgen05 kernel at any number of distinct rows
+    const bool tensor = !(flags & BMM_FLAG_NO_TENSOR) && bmm::waic_tc_supported(K, P) &&
+                        ((force && force[0] == '1') || (long long)ntc >= (long long)WAIC_TC_MIN_TILES_PER_SM * sms);
+    DevBuf rb, wd, th, pd, tab, img, bias, stat, tpart, lp, pw, cv, ll, ct, sd;
+    TRY(upload(rb, rowbits.data(), rowbits.size()));
+    TRY(upload(wd, wt.data(), wt.size()));
+    TRY(upload(th, theta, (size_t)D * K * P));
+    TRY(upload(pd, pid.data(), pid.size()));
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    CU(cudaEventCreate(&e0));
+    CU(cudaEventCreate(&e1));
+    struct EvPair { cudaEvent_t a, b; ~EvPair() { cudaEventDestroy(a); cudaEventDestroy(b); } } evs{e0, e1};
+    int Q;
+    long long G;
+    CU(cudaEventRecord(e0, 0));
+    if (tensor) {
+        Q = 1;
+        G = 4LL * ntc;
+        CU(img.alloc((size_t)D * bmm::waic_tc_img_bytes(P), false));
+        CU(bias.alloc((size_t)D * 32 * 4, false));
+        CU(sd.alloc(4));
+        CU(stat.alloc((size_t)C * U * bmm::WAIC_STAT * 8, false));
+        CU(tpart.alloc((size_t)D * G * 8, false));
+        CU(bmm::launch_waic_tc_tables(K, P, D, th.as<double>(), pd.as<double>(), img.as<unsigned char>(), bias.as<float>(), 0));
+        CU(bmm::launch_waic_tc(U, P, W, K, S, C, rb.as<uint32_t>(), wd.as<int>(), img.as<unsigned char>(), bias.as<float>(),
+                               stat.as<double>(), tpart.as<double>(), sd.as<int>(), sms, 0));
+    } else {
+        const int nt = (U + 31) / 32;
+        const int q0 = bmm::waic_fp64_slices(nt, C, S), SL = (S + q0 - 1) / q0;
+        Q = (S + SL - 1) / SL;                               // slices of SL = ceil(S / Q) draws, none empty
+        G = nt;
+        CU(tab.alloc((size_t)D * K * (2 * P + 1) * 8, false));
+        CU(stat.alloc((size_t)C * Q * U * bmm::WAIC_STAT * 8, false));
+        CU(tpart.alloc((size_t)D * G * 8, false));
+        CU(bmm::launch_predict_tables(K, P, (int)D, th.as<double>(), pd.as<double>(), tab.as<double>(), 0));
+        CU(bmm::launch_waic_fp64(U, P, W, K, S, C, Q, rb.as<uint32_t>(), wd.as<int>(), tab.as<double>(), stat.as<double>(),
+                                 tpart.as<double>(), 0));
+    }
+    CU(lp.alloc((size_t)U * 8, false));
+    CU(pw.alloc((size_t)U * 8, false));
+    CU(cv.alloc((size_t)2 * C * U * 8, false));
+    CU(ll.alloc((size_t)D * 8, false));
+    CU(ct.alloc((size_t)2 * C * 8, false));
+    CU(bmm::launch_waic_merge(U, C, S, Q, wd.as<int>(), stat.as<double>(), G, tpart.as<double>(), lp.as<double>(),
+                              pw.as<double>(), cv.as<double>(), ll.as<double>(), ct.as<double>(), 0));
+    CU(cudaEventRecord(e1, 0));
+    CU(cudaEventSynchronize(e1));
+    CU(cudaEventElapsedTime(&g_waic_ms, e0, e1));
+    g_waic_tensor = tensor;
+    if (tensor) {
+        int st = 0;
+        CU(cudaMemcpy(&st, sd.p, 4, cudaMemcpyDeviceToHost));
+        if (st) return fail(st, "waic tensor kernel: an mbarrier wait timed out");
+    }
+    if (loglik) CU(cudaMemcpy(loglik, ll.p, (size_t)D * 8, cudaMemcpyDeviceToHost));
+    if (chain_lppd) CU(cudaMemcpy(chain_lppd, ct.p, (size_t)C * 8, cudaMemcpyDeviceToHost));
+    if (chain_p_waic) CU(cudaMemcpy(chain_p_waic, ct.as<double>() + C, (size_t)C * 8, cudaMemcpyDeviceToHost));
+    if (lppd || p_waic) {
+        std::vector<double> ul(U), up(U);
+        CU(cudaMemcpy(ul.data(), lp.p, (size_t)U * 8, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(up.data(), pw.p, (size_t)U * 8, cudaMemcpyDeviceToHost));
+        for (int i = 0; i < N; ++i) {
+            if (lppd) lppd[i] = ul[rowid[i]];
+            if (p_waic) p_waic[i] = up[rowid[i]];
+        }
+    }
+    return BMM_OK;
+}
+
+int bmm_waic_kernel_ms(float *ms, int32_t *tensor) {
+    if (!ms || !tensor) return fail(BMM_ERR_INVALID, "ms / tensor is NULL");
+    *ms = g_waic_ms;
+    *tensor = g_waic_tensor;
     return BMM_OK;
 }
 

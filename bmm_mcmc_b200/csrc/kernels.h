@@ -1,5 +1,6 @@
 // Host-visible parameter blocks and launchers of the sampler kernels.
 #pragma once
+#include <cmath>
 #include <cstdint>
 #include <cuda_runtime.h>
 
@@ -289,6 +290,52 @@ cudaError_t launch_rdirichlet(int K, const double *alpha_m, unsigned long long s
 // tab: scratch of S * K * (2 P + 1) doubles; member (optional, zeroed by the caller): M x K column-major
 cudaError_t launch_predict(int M, int P, int W, int K, int S, const uint32_t *xbits, const double *theta, const double *pi,
                            double *tab, double *logpred, double *member, cudaStream_t st);
+// tab[g][k][0..P) = log theta_kd, [P..2P) = log(1 - theta_kd), [2P] = log pi_k of S draws (theta K x P x S, pi S x K cm)
+cudaError_t launch_predict_tables(int K, int P, int S, const double *theta, const double *pi, double *tab, cudaStream_t st);
+
+// ---- WAIC and the log-likelihood trace (kern_predict.cu fp64, kern_waic_tc.cu tcgen05) ---------------------------------
+// Mergeable partials of one row over a run of draws: n, mean, M2 (Welford) and max, sum (log-sum-exp of l).
+constexpr int WAIC_STAT = 5;
+__host__ __device__ inline void waic_stat_init(double (&a)[WAIC_STAT]) { a[0] = a[1] = a[2] = a[4] = 0.0; a[3] = -INFINITY; }
+__host__ __device__ inline void waic_stat_merge(double (&a)[WAIC_STAT], const double *b) {
+    if (b[0] == 0.0) return;
+    if (a[0] == 0.0) { for (int e = 0; e < WAIC_STAT; ++e) a[e] = b[e]; return; }
+    const double na = a[0], nb = b[0], n = na + nb, delta = b[1] - a[1];   // Chan, Golub & LeVeque (1979)
+    a[1] += delta * (nb / n);
+    a[2] += b[2] + delta * delta * (na * nb / n);
+    a[0] = n;
+    if (b[4] > 0.0) {
+        if (b[3] > a[3]) { a[4] = a[4] * exp(a[3] - b[3]) + b[4]; a[3] = b[3]; }
+        else a[4] += b[4] * exp(b[3] - a[3]);
+    }
+}
+// one more draw's l
+__host__ __device__ inline void waic_push(double (&st)[WAIC_STAT], double l) {
+    st[0] += 1.0;
+    const double delta = l - st[1];
+    st[1] += delta / st[0];
+    st[2] += delta * (l - st[1]);
+    if (l > st[3]) { st[4] = st[4] * exp(st[3] - l) + 1.0; st[3] = l; }
+    else if (l > -INFINITY) st[4] += exp(l - st[3]);
+}
+// slices per chain of the fp64 kernel for ntiles tiles of 32 distinct rows
+int waic_fp64_slices(int ntiles, int C, int S);
+// stat: [C Q][U][WAIC_STAT]; tpart: [C S][ceil(U / 32)]; tab from launch_predict_tables over the C S draws
+cudaError_t launch_waic_fp64(int U, int P, int W, int K, int S, int C, int Q, const uint32_t *rowbits, const int *wt,
+                             const double *tab, double *stat, double *tpart, cudaStream_t st);
+// pooled pointwise lppd / p_waic [U]; cv scratch [2 C][U]; loglik [C S] = sum of the G trace partials of each draw
+// (tpart [C S][G]); chain_tot [2 C] = per-chain lppd, then per-chain p_waic (multiplicity-weighted sums over rows)
+cudaError_t launch_waic_merge(int U, int C, int S, int Q, const int *wt, const double *stat, long long G, const double *tpart,
+                              double *lppd, double *pwaic, double *cv, double *loglik, double *chain_tot, cudaStream_t st);
+// tcgen05 path, K <= 32 and P <= 112: img [C S][ws_nch(P) * WS_B1_ROW] operand images and bias [C S][32] (log2 units),
+// built by launch_waic_tc_tables; stat [C][U][WAIC_STAT] (one slice per chain); tpart [C S][4 ceil(U / 128)]
+bool waic_tc_supported(int K, int P);
+size_t waic_tc_img_bytes(int P);
+cudaError_t launch_waic_tc_tables(int K, int P, long long D, const double *theta, const double *pi, unsigned char *img,
+                                  float *bias, cudaStream_t st);
+cudaError_t launch_waic_tc(int U, int P, int W, int K, int S, int C, const uint32_t *rowbits, const int *wt,
+                           const unsigned char *img, const float *bias, double *stat, double *tpart, int *status,
+                           int sm_count, cudaStream_t st);
 
 // ---- history layout conversion (kern_finalize.cu) --------------------------------------------
 // zhist [c][nsamples][N] uint8 -> R layout [c][S x N cm]; optional relabelling through perm_out.

@@ -51,7 +51,8 @@ extern "C" {
                                         uint32 [N][ceil(P/32)], bit d%32 of word d/32 = x_id (grid
                                         path only; 8 B per row at P = 64 instead of 256 B)         */
 #define BMM_FLAG_NO_TENSOR 32u        /* grid path, BMM_FP32: use the CUDA-core float kernel instead of
-                                        the tcgen05 contraction (A/B testing)                      */
+                                        the tcgen05 contraction (A/B testing); bmm_waic: the fp64
+                                        kernel                                                     */
 #define BMM_FLAG_STEPHENS_FIXED 64u   /* correctness-fixed relabelling (NOT the reference, SURVEY 8f-3): the batch
                                       * initialisation and the online Q update re-order columns with the
                                       * inverse of index_max(solution.col(.)) -- what the no-op
@@ -182,6 +183,23 @@ int bmm_rdirichlet(int32_t K, const double *alpha_m, uint64_t seed, double *out)
  * membership (optional, M x K column-major) = the responsibilities averaged over the draws.             */
 int bmm_predictive(const int32_t *Xnew, int32_t M, int32_t P, int32_t K, int32_t S, const double *theta, const double *pi,
                    double *log_pred, double *membership);
+/* WAIC (Watanabe 2010; as R's loo::waic) and the observed-data log-likelihood trace of a fitted gibbs_full /
+ * gibbs_stickbreaking model (no reference counterpart).  X: N x P int32 column-major 0/1, or with BMM_FLAG_X_PACKED
+ * uint32 [N][ceil(P/32)] bit-packed rows.  theta [C][K x P x S] and pi [C][S x K cm]: the kept draws of C chains as the
+ * samplers return them.  With l[c,s,i] = log sum_k pi_k prod_d theta_kd^x_id (1 - theta_kd)^(1 - x_id) of draw (c, s):
+ *   loglik [C x S]        sum_i l[c,s,i]
+ *   lppd [N]              log 1/(C S) sum_{c,s} exp l[c,s,i]
+ *   p_waic [N]            variance of l[.,.,i] over the C S draws, denominator C S - 1
+ *   chain_lppd [C], chain_p_waic [C]   the totals over i of the same two figures from chain c's S draws alone
+ * Any output may be NULL.  C S >= 2.  Computed on the device in a fixed order (two calls return the same bits): the fp64
+ * kernel, or for K <= 32, P <= 112 and enough distinct rows a tcgen05 kernel (fp16 hi|lo operands, fp32 log-sum-exp over
+ * k, fp64 moments); BMM_FLAG_NO_TENSOR forces the fp64 kernel.  theta exactly 0 or 1 gives l = -inf on the fp64 kernel,
+ * and then p_waic = nan, as the float64 definition does.                                                          */
+int bmm_waic(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta, const double *pi,
+             uint32_t flags, int32_t device, double *loglik, double *lppd, double *p_waic, double *chain_lppd,
+             double *chain_p_waic);
+/* Device time in ms of the last bmm_waic's kernels on this thread, and 1 if it took the tcgen05 kernel.               */
+int bmm_waic_kernel_ms(float *ms, int32_t *tensor);
 
 /* Diagnostic (no reference counterpart): %globaltimer stamps in ns of the last two sweeps of the tensor grid path.
  * out[8 * (j & 1) + s], z-sweep kernel CTA 0: s = 0 entry, 1 pipeline start, 2 first tile drawn, 3 last tile drawn,

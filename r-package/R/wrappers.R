@@ -70,3 +70,23 @@ predict_gibbs <- function(obj, newdata) {
     storage.mode(newdata) <- "integer"
     predictive_cpp(newdata, obj$theta, obj$pi)
 }
+
+#' WAIC of a fitted model
+#'
+#' Not in the reference: the widely applicable information criterion (Watanabe 2010) of an uncollapsed fit, computed on
+#' the GPU, in the layout of \code{loo::waic}, to compare fits at several K (lower \code{waic} is better).
+#'
+#' @param obj The list returned by \code{gibbs_full} or \code{gibbs_stickbreaking}.
+#' @param data The N x P 0/1 matrix the model was fitted to.
+#' @return A list with \code{estimates} (rows elpd_waic, p_waic, waic; columns Estimate, SE), \code{pointwise}
+#'   (N x 3, the same three columns) and \code{loglik}, the observed-data log-likelihood of every kept draw.
+#' @export
+waic_gibbs <- function(obj, data) {
+    if (is.null(obj$pi)) stop("waic_gibbs needs the pi history of gibbs_full / gibbs_stickbreaking")
+    data <- as.matrix(data)
+    storage.mode(data) <- "integer"
+    r <- waic_cpp(data, obj$theta, obj$pi)
+    dimnames(r$estimates) <- list(c("elpd_waic", "p_waic", "waic"), c("Estimate", "SE"))
+    colnames(r$pointwise) <- c("elpd_waic", "p_waic", "waic")
+    r
+}

@@ -7,6 +7,8 @@
 // The build image has no R / Rcpp: tests/test_rhost.py compiles this file, unmodified, against the Rcpp stand-in of
 // oracle/shim/ and checks on the GPU that every element of the returned lists equals the ctypes path's.  Everything
 // below the C ABI is exercised through the same entry points by tests/test_gpu_parity.py.
+#include <cmath>
+
 #include <Rcpp.h>
 
 #include "bmm_capi.h"
@@ -146,6 +148,37 @@ NumericMatrix rdirichlet_cpp(NumericVector alpha_m) {
     NumericMatrix out(K, 1);                       // arma::vec wraps as a K x 1 matrix in the reference
     if (bmm_rdirichlet(K, alpha_m.begin(), philox_seed(), out.begin()) != BMM_OK) stop(bmm_last_error());
     return out;
+}
+
+// WAIC of a fitted model (no reference counterpart; the layout of loo::waic): estimates 3 x 2 (rows elpd_waic, p_waic, waic;
+// columns Estimate, SE = sqrt(N var(pointwise))), pointwise N x 3 (same columns order as the estimate rows), loglik[S].
+// theta: K x P x S array and pi: S x K matrix as gibbs_full / gibbs_stickbreaking return them; data: the N x P 0/1 matrix.
+// [[Rcpp::export]]
+List waic_cpp(IntegerMatrix data, NumericVector theta, NumericMatrix pi) {
+    IntegerVector dim = theta.attr("dim");
+    if (dim.size() != 3) stop("theta must be a K x P x S array");
+    const int K = dim[0], P = dim[1], S = dim[2], N = data.nrow();
+    if (data.ncol() != P || pi.nrow() != S || pi.ncol() != K) stop("data / theta / pi dimensions do not match");
+    if (S < 2) stop("waic needs at least 2 draws");
+    NumericVector loglik(S), lppd(N), pw(N);
+    if (bmm_waic(data.begin(), N, P, K, S, 1, theta.begin(), pi.begin(), 0u, 0, loglik.begin(), lppd.begin(), pw.begin(),
+                 nullptr, nullptr) != BMM_OK)
+        stop(bmm_last_error());
+    NumericMatrix pointwise(N, 3), estimates(3, 2);
+    for (int i = 0; i < N; ++i) {
+        pointwise(i, 0) = lppd[i] - pw[i];
+        pointwise(i, 1) = pw[i];
+        pointwise(i, 2) = -2.0 * (lppd[i] - pw[i]);
+    }
+    for (int j = 0; j < 3; ++j) {
+        double sum = 0.0, ss = 0.0;
+        for (int i = 0; i < N; ++i) sum += pointwise(i, j);
+        const double mean = sum / N;
+        for (int i = 0; i < N; ++i) ss += (pointwise(i, j) - mean) * (pointwise(i, j) - mean);
+        estimates(j, 0) = sum;
+        estimates(j, 1) = N > 1 ? std::sqrt(N * (ss / (N - 1))) : NAN;
+    }
+    return List::create(Named("estimates") = estimates, Named("pointwise") = pointwise, Named("loglik") = loglik);
 }
 
 // Posterior predictive distribution (no reference counterpart; the reference's TODO:6 lists it).  theta: K x P x S array
