@@ -17,7 +17,8 @@ import numpy as np
 from . import _lib
 from .rcompat import RRng
 
-__all__ = ["gibbs_full", "gibbs_collapsed", "gibbs_dp", "gibbs_stickbreaking", "predictive", "waic", "Plan", "PackedX"]
+__all__ = ["gibbs_full", "gibbs_collapsed", "gibbs_dp", "gibbs_stickbreaking", "predictive", "waic", "loo", "loglik_matrix", "Plan",
+           "PackedX"]
 
 
 def _r_round(x):
@@ -436,6 +437,20 @@ def _waic_draws(fit):
             Cn, K, P, S, chains)
 
 
+def _loglik_inputs(fit, data, no_tensor, what):
+    """The C ABI's arguments shared by waic(), loo() and loglik_matrix(), checked on the host.  X is returned with its
+    address: the caller keeps it alive across the library call."""
+    th, pi, Cn, K, P, S, chains = _waic_draws(fit)
+    X = _as_X(data)
+    if X.shape[1] != P:
+        raise ValueError("data has %d columns, theta has %d variables" % (X.shape[1], P))
+    if Cn * S < 2:
+        raise ValueError("%s needs at least 2 draws" % what)
+    flags = (_lib.FLAG_X_PACKED if isinstance(X, PackedX) else 0) | (_lib.FLAG_NO_TENSOR if no_tensor else 0)
+    xp = X.bits.ctypes.data if isinstance(X, PackedX) else X.ctypes.data
+    return th, pi, Cn, K, P, S, chains, X, flags, C.c_void_p(xp)
+
+
 def waic(fit, data, *, no_tensor=False, device=0):
     """WAIC of a fitted `gibbs_full` / `gibbs_stickbreaking` model and the log-likelihood trace of its draws, computed on the
     device (Watanabe 2010; Vehtari, Gelman & Gabry 2017, the layout of R's `loo::waic`).
@@ -448,19 +463,12 @@ def waic(fit, data, *, no_tensor=False, device=0):
 
     K <= 32 and P <= 112 fits with many distinct rows run on the tcgen05 kernel (fp16 hi|lo operands, fp32 log-sum-exp,
     fp64 moments); `no_tensor=True` forces the fp64 kernel."""
-    th, pi, Cn, K, P, S, chains = _waic_draws(fit)
-    X = _as_X(data)
+    th, pi, Cn, K, P, S, chains, X, flags, xp = _loglik_inputs(fit, data, no_tensor, "waic")
     N = X.shape[0]
-    if X.shape[1] != P:
-        raise ValueError("data has %d columns, theta has %d variables" % (X.shape[1], P))
-    if Cn * S < 2:
-        raise ValueError("waic needs at least 2 draws")
-    flags = (_lib.FLAG_X_PACKED if isinstance(X, PackedX) else 0) | (_lib.FLAG_NO_TENSOR if no_tensor else 0)
     ll = np.zeros((Cn, S))
     lppd, pw = np.zeros(N), np.zeros(N)
     clp, cpw = np.zeros(Cn), np.zeros(Cn)
-    xp = X.bits.ctypes.data if isinstance(X, PackedX) else X.ctypes.data
-    _lib.check(_lib.lib().bmm_waic(C.c_void_p(xp), N, P, K, S, Cn, _p(th, C.c_double), _p(pi, C.c_double), flags,
+    _lib.check(_lib.lib().bmm_waic(xp, N, P, K, S, Cn, _p(th, C.c_double), _p(pi, C.c_double), flags,
                                    int(device), _p(ll, C.c_double), _p(lppd, C.c_double), _p(pw, C.c_double),
                                    _p(clp, C.c_double), _p(cpw, C.c_double)))
     elpd = lppd - pw
@@ -475,3 +483,60 @@ def waic(fit, data, *, no_tensor=False, device=0):
         out["chain_waic"] = -2.0 * (clp - cpw)
         out["chain_p_waic"] = cpw
     return out
+
+
+def loo(fit, data, *, r_eff=1.0, no_tensor=False, device=0):
+    """PSIS-LOO of a fitted `gibbs_full` / `gibbs_stickbreaking` model, computed on the device (Vehtari, Gelman & Gabry
+    2017; the algorithm and the layout of R's `loo::loo`, without `mcse_elpd_loo`).
+
+    `data` is the N x P 0/1 matrix the model was fitted to, or a `PackedX`; with a chain axis the C chains' S draws are
+    pooled (D = C S >= 2).  `r_eff` (a scalar or N values, finite and > 0) is the relative efficiency of each observation's
+    draws: it sets the Pareto tail length min(ceil(0.2 D), ceil(3 sqrt(D / r_eff))) and scales `n_eff`; computing it
+    from the chains (`loo::relative_eff`) is left to the caller.  Returns the pointwise arrays `pointwise_elpd_loo`,
+    `pointwise_lpd` (= waic()'s lppd), `pointwise_p_loo` = lpd - elpd_loo and `pointwise_looic` = -2 elpd_loo; their
+    totals and `se_*` = sqrt(N var_i(pointwise)); `pareto_k` (inf where the tail has fewer than 5 draws or is flat) and
+    `n_eff` per observation; `k_threshold` = min(1 - 1 / log10(D), 0.7) and the counts of observations with k at most
+    the threshold (`n_k_good`), in (threshold, 1] (`n_k_bad`) and above 1 (`n_k_very_bad`, where the estimate cannot
+    be trusted).
+
+    The log-likelihood matrix comes from the tcgen05 kernel for K <= 32, P <= 112 fits with many distinct rows (as in
+    waic()); `no_tensor=True` forces the fp64 kernel.  The smoothing and the sums run in fp64."""
+    th, pi, Cn, K, P, S, chains, X, flags, xp = _loglik_inputs(fit, data, no_tensor, "loo")
+    N = X.shape[0]
+    re = np.asarray(r_eff, dtype=np.float64)
+    if re.ndim == 0:
+        re = np.full(N, float(re))
+    if re.shape != (N,):
+        raise ValueError("r_eff must be a scalar or have one value per observation (%d)" % N)
+    if not (np.isfinite(re).all() and (re > 0).all()):
+        raise ValueError("r_eff must be finite and > 0")
+    re = np.ascontiguousarray(re)
+    elpd, lpd, k, neff = np.zeros(N), np.zeros(N), np.zeros(N), np.zeros(N)
+    _lib.check(_lib.lib().bmm_loo(xp, N, P, K, S, Cn, _p(th, C.c_double), _p(pi, C.c_double), _p(re, C.c_double), flags,
+                                  int(device), _p(elpd, C.c_double), _p(lpd, C.c_double), _p(k, C.c_double),
+                                  _p(neff, C.c_double)))
+    out = {"pointwise_elpd_loo": elpd, "pointwise_lpd": lpd, "pointwise_p_loo": lpd - elpd, "pointwise_looic": -2.0 * elpd}
+    for name in ("elpd_loo", "lpd", "p_loo", "looic"):
+        v = out["pointwise_" + name]
+        out[name] = float(v.sum())
+        out["se_" + name] = float(np.sqrt(N * np.var(v, ddof=1))) if N > 1 else float("nan")
+    out["pareto_k"], out["n_eff"] = k, neff
+    D = Cn * S
+    thr = min(1.0 - 1.0 / np.log10(D), 0.7)
+    out["k_threshold"] = thr
+    out["n_k_good"] = int(np.sum(k <= thr))
+    out["n_k_bad"] = int(np.sum((k > thr) & (k <= 1)))
+    out["n_k_very_bad"] = int(np.sum(k > 1))
+    return out
+
+
+def loglik_matrix(fit, data, *, no_tensor=False, device=0):
+    """l[g, i] = log p(x_i | draw g) of a fitted `gibbs_full` / `gibbs_stickbreaking` model, computed on the device: a
+    D x N array over the S kept draws, or C x S x N when the fit has a chain axis (the matrix / array `loo::loo()` takes).
+    The kernels and `no_tensor` are those of loo()."""
+    th, pi, Cn, K, P, S, chains, X, flags, xp = _loglik_inputs(fit, data, no_tensor, "loglik_matrix")
+    N = X.shape[0]
+    out = np.zeros((N, Cn * S))
+    _lib.check(_lib.lib().bmm_loglik_matrix(xp, N, P, K, S, Cn, _p(th, C.c_double), _p(pi, C.c_double), flags, int(device),
+                                            _p(out, C.c_double)))
+    return out.T.reshape(Cn, S, N) if chains else out.T

@@ -12,7 +12,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libbmm_b200.so")
 SOURCES = ["capi.cu", "dist.cu", "kern_full.cu", "kern_collapsed.cu", "kern_stephens.cu", "kern_finalize.cu",
-           "kern_big.cu", "kern_big_ws.cu", "kern_big_lp.cu", "kern_big_counts.cu", "kern_big_relabel.cu", "kern_big_cost_tc.cu", "kern_big_ws_relabel.cu", "kern_predict.cu", "kern_waic_tc.cu",
+           "kern_big.cu", "kern_big_ws.cu", "kern_big_lp.cu", "kern_big_counts.cu", "kern_big_relabel.cu", "kern_big_cost_tc.cu", "kern_big_ws_relabel.cu", "kern_predict.cu", "kern_waic_tc.cu", "kern_loo.cu",
            "host_widen.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",

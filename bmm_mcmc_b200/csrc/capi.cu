@@ -1516,6 +1516,36 @@ static thread_local float g_waic_ms = 0.f;
 static thread_local int32_t g_waic_tensor = 0;
 static constexpr int WAIC_TC_MIN_TILES_PER_SM = 1;
 
+// X as bit-packed rows [N][W]: packs an int32 N x P column-major 0/1 matrix, or copies BMM_FLAG_X_PACKED rows with the
+// bits beyond P cleared (they are not part of the row)
+static int input_rows(const void *X, int N, int P, uint32_t flags, std::vector<uint32_t> &bits, int &W) {
+    W = (P + 31) / 32;
+    if (flags & BMM_FLAG_X_PACKED) {
+        const uint32_t *xb = (const uint32_t *)X, tail = (P & 31) ? (1u << (P & 31)) - 1u : ~0u;
+        bits.assign(xb, xb + (size_t)N * W);
+        for (int i = 0; i < N; ++i) bits[(size_t)i * W + W - 1] &= tail;
+        return BMM_OK;
+    }
+    return pack_rows((const int32_t *)X, N, P, bits, W);
+}
+
+// pi [C][S x K cm] -> D x K cm over the chain-major draws g = c S + s (theta [C][K x P x S] already is K x P x D)
+static std::vector<double> pooled_pi(const double *pi, int C, int S, int K) {
+    const size_t D = (size_t)C * S;
+    std::vector<double> pid(D * K);
+    for (int c = 0; c < C; ++c)
+        for (int k = 0; k < K; ++k)
+            for (int s = 0; s < S; ++s) pid[(size_t)c * S + s + D * k] = pi[(size_t)c * S * K + s + (size_t)S * k];
+    return pid;
+}
+
+// the tcgen05 kernels take the shapes they cover once there are U distinct rows enough to give every SM a 128-row tile
+static bool waic_tensor_path(uint32_t flags, int K, int P, int U, int sms) {
+    const char *force = getenv("BMM_WAIC_TENSOR");   // tests: the tcgen05 kernel at any number of distinct rows
+    return !(flags & BMM_FLAG_NO_TENSOR) && bmm::waic_tc_supported(K, P) &&
+           ((force && force[0] == '1') || (long long)(U + 127) / 128 >= (long long)WAIC_TC_MIN_TILES_PER_SM * sms);
+}
+
 int bmm_waic(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta, const double *pi,
              uint32_t flags, int32_t device, double *loglik, double *lppd, double *p_waic, double *chain_lppd,
              double *chain_p_waic) {
@@ -1526,31 +1556,19 @@ int bmm_waic(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t 
     if (D > 0x7FFFFFFFLL) return fail(BMM_ERR_INVALID, "waic: C * S too large");
     if (device < 0 || bmm_device_count() <= device) return fail(BMM_ERR_CUDA, "no CUDA device (this library has no CPU fallback)");
     std::vector<uint32_t> bits;
-    int W = (P + 31) / 32;
-    if (flags & BMM_FLAG_X_PACKED) {
-        const uint32_t *xb = (const uint32_t *)X, tail = (P & 31) ? (1u << (P & 31)) - 1u : ~0u;
-        bits.assign(xb, xb + (size_t)N * W);
-        for (int i = 0; i < N; ++i) bits[(size_t)i * W + W - 1] &= tail;   // bits beyond P are not part of the row
-    } else {
-        TRY(pack_rows((const int32_t *)X, N, P, bits, W));
-    }
+    int W;
+    TRY(input_rows(X, N, P, flags, bits, W));
     std::vector<int> rowid, wt;
     std::vector<uint32_t> rowbits;
     dedup_rows(bits.data(), N, W, rowid, wt, rowbits);
     std::vector<uint32_t>().swap(bits);
     const int U = (int)wt.size();
-    // pi [C][S x K cm] -> D x K cm over the chain-major draws g = c S + s (theta [C][K x P x S] already is K x P x D)
-    std::vector<double> pid((size_t)D * K);
-    for (int c = 0; c < C; ++c)
-        for (int k = 0; k < K; ++k)
-            for (int s = 0; s < S; ++s) pid[(size_t)c * S + s + (size_t)D * k] = pi[(size_t)c * S * K + s + (size_t)S * k];
+    const std::vector<double> pid = pooled_pi(pi, C, S, K);
     CU(cudaSetDevice(device));
     int sms = 0;
     CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     const int ntc = (U + 127) / 128;
-    const char *force = getenv("BMM_WAIC_TENSOR");   // tests: the tcgen05 kernel at any number of distinct rows
-    const bool tensor = !(flags & BMM_FLAG_NO_TENSOR) && bmm::waic_tc_supported(K, P) &&
-                        ((force && force[0] == '1') || (long long)ntc >= (long long)WAIC_TC_MIN_TILES_PER_SM * sms);
+    const bool tensor = waic_tensor_path(flags, K, P, U, sms);
     DevBuf rb, wd, th, pd, tab, img, bias, stat, tpart, lp, pw, cv, ll, ct, sd;
     TRY(upload(rb, rowbits.data(), rowbits.size()));
     TRY(upload(wd, wt.data(), wt.size()));
@@ -1621,6 +1639,234 @@ int bmm_waic_kernel_ms(float *ms, int32_t *tensor) {
     if (!ms || !tensor) return fail(BMM_ERR_INVALID, "ms / tensor is NULL");
     *ms = g_waic_ms;
     *tensor = g_waic_tensor;
+    return BMM_OK;
+}
+
+// PSIS-LOO and the log-likelihood matrix (kern_loo.cu).  Both read l[g, u] of the distinct rows from one device buffer
+// that holds a chunk of rows at a time: the smaller of LOGLIK_CHUNK_CAP bytes and a quarter of the free device memory
+// (the whole C4 matrix would take 7.2 GB).  BMM_LOO_CHUNK_ROWS caps the rows of a chunk (tests: many chunks).
+static thread_local float g_loo_ms = 0.f;
+static thread_local int32_t g_loo_tensor = 0;
+static constexpr size_t LOGLIK_CHUNK_CAP = (size_t)2 << 30;
+
+// The draws' tables and the matrix producer: L [D][uc] <- l of distinct rows [u0, u0 + uc), fp64 or tcgen05 kernel
+struct LoglikMat {
+    long long D = 0;
+    int U = 0, W = 0, P = 0, K = 0, sms = 0, rows = 0;   // rows: the chunk size
+    bool tensor = false;
+    DevBuf rb, th, pd, tab, img, bias, sd, L;
+
+    int init(const std::vector<uint32_t> &rowbits, int U_, int W_, int P_, int K_, int S, int C, const double *theta,
+             const double *pi, uint32_t flags, int device) {
+        U = U_; W = W_; P = P_; K = K_;
+        D = (long long)C * S;
+        CU(cudaSetDevice(device));
+        CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+        tensor = waic_tensor_path(flags, K, P, U, sms);
+        const std::vector<double> pid = pooled_pi(pi, C, S, K);
+        TRY(upload(rb, rowbits.data(), rowbits.size()));
+        TRY(upload(th, theta, (size_t)D * K * P));
+        TRY(upload(pd, pid.data(), pid.size()));
+        size_t fre = 0, tot = 0;
+        CU(cudaMemGetInfo(&fre, &tot));
+        long long r = (long long)(std::min(LOGLIK_CHUNK_CAP, fre / 4) / ((size_t)D * 8));
+        if (const char *e = getenv("BMM_LOO_CHUNK_ROWS")) { const long long c = atoll(e); if (c > 0 && r > c) r = c; }
+        rows = (int)std::max(1LL, std::min(r, (long long)U));
+        CU(L.alloc((size_t)rows * D * 8, false));
+        if (tensor) {
+            CU(img.alloc((size_t)D * bmm::waic_tc_img_bytes(P), false));
+            CU(bias.alloc((size_t)D * 32 * 4, false));
+            CU(sd.alloc(4));
+        } else {
+            CU(tab.alloc((size_t)D * K * (2 * P + 1) * 8, false));
+        }
+        return BMM_OK;
+    }
+    int tables() {
+        if (tensor)
+            CU(bmm::launch_waic_tc_tables(K, P, D, th.as<double>(), pd.as<double>(), img.as<unsigned char>(), bias.as<float>(), 0));
+        else
+            CU(bmm::launch_predict_tables(K, P, (int)D, th.as<double>(), pd.as<double>(), tab.as<double>(), 0));
+        return BMM_OK;
+    }
+    int produce(int u0, int n) {
+        const uint32_t *xb = rb.as<uint32_t>() + (size_t)u0 * W;
+        if (tensor)
+            CU(bmm::launch_loglik_tc(n, P, W, D, xb, img.as<unsigned char>(), bias.as<float>(), L.as<double>(), sd.as<int>(), sms, 0));
+        else
+            CU(bmm::launch_loglik_fp64(n, P, W, K, D, xb, tab.as<double>(), L.as<double>(), 0));
+        return BMM_OK;
+    }
+    int status() {
+        if (!tensor) return BMM_OK;
+        int st = 0;
+        CU(cudaMemcpy(&st, sd.p, 4, cudaMemcpyDeviceToHost));
+        return st ? fail(st, "log-likelihood tensor kernel: an mbarrier wait timed out") : BMM_OK;
+    }
+};
+
+static int loglik_args(const void *X, int N, int P, int K, int S, int C, const double *theta, const double *pi,
+                       const char *what) {
+    if (!X || !theta || !pi || N < 1 || P < 1 || K < 1 || K > 255 || S < 1 || C < 1)
+        return fail(BMM_ERR_INVALID, std::string("bad ") + what + " arguments");
+    const long long D = (long long)C * S;
+    if (D < 2) return fail(BMM_ERR_INVALID, std::string(what) + " needs at least 2 draws (C * S >= 2)");
+    if (D > 0x7FFFFFFFLL) return fail(BMM_ERR_INVALID, std::string(what) + ": C * S too large");
+    return BMM_OK;
+}
+
+int bmm_loo(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta, const double *pi,
+            const double *r_eff, uint32_t flags, int32_t device, double *elpd_loo, double *lpd, double *pareto_k,
+            double *n_eff) {
+    TRY(loglik_args(X, N, P, K, S, C, theta, pi, "loo"));
+    const long long D = (long long)C * S;
+    // tail length of each observation, loo's n_pareto_tail; no smoothing below 5
+    std::vector<int> Mi(N);
+    for (int i = 0; i < N; ++i) {
+        const double re = r_eff ? r_eff[i] : 1.0;
+        if (!(re > 0.0) || !std::isfinite(re)) return fail(BMM_ERR_INVALID, "loo: r_eff must be finite and > 0");
+        const double m = std::min(std::ceil(0.2 * (double)D), std::ceil(3 * std::sqrt((double)D / re)));
+        if (m > bmm::LOO_MAX_TAIL) {
+            char msg[256];
+            snprintf(msg, sizeof msg, "loo: the Pareto tail of %lld draws at r_eff = %g has %.0f draws; at most %d are supported "
+                     "(D <= 29826161 at r_eff = 1)", D, re, m, bmm::LOO_MAX_TAIL);
+            return fail(BMM_ERR_INVALID, msg);
+        }
+        Mi[i] = (int)m;
+    }
+    if (device < 0 || bmm_device_count() <= device) return fail(BMM_ERR_CUDA, "no CUDA device (this library has no CPU fallback)");
+    std::vector<uint32_t> bits;
+    int W;
+    TRY(input_rows(X, N, P, flags, bits, W));
+    // de-duplicate on (row, M): r_eff changes only the tail length, and n_eff's r_eff factor is applied per observation
+    std::vector<uint32_t> keys((size_t)N * (W + 1));
+    for (int i = 0; i < N; ++i) {
+        std::memcpy(&keys[(size_t)i * (W + 1)], &bits[(size_t)i * W], (size_t)W * 4);
+        keys[(size_t)i * (W + 1) + W] = (uint32_t)Mi[i];
+    }
+    std::vector<uint32_t>().swap(bits);
+    std::vector<int> rowid, wt;
+    std::vector<uint32_t> urows;
+    dedup_rows(keys.data(), N, W + 1, rowid, wt, urows);
+    std::vector<uint32_t>().swap(keys);
+    const int U = (int)wt.size();
+    std::vector<uint32_t> rowbits((size_t)U * W);
+    std::vector<int> Mu(U);
+    for (int u = 0; u < U; ++u) {
+        std::memcpy(&rowbits[(size_t)u * W], &urows[(size_t)u * (W + 1)], (size_t)W * 4);
+        Mu[u] = (int)urows[(size_t)u * (W + 1) + W];
+    }
+    LoglikMat lm;
+    TRY(lm.init(rowbits, U, W, P, K, S, C, theta, pi, flags, device));
+    // per chunk: the long-tail rows (chunk-local index, M, offset into the chunk's tail storage) and the widest tails
+    const int rows = lm.rows, nch = (U + rows - 1) / rows;
+    std::vector<int> lrow, lM, l0(nch + 1), short_m(nch, 0), long_m(nch, 0);
+    std::vector<long long> ltoff;
+    long long max_tail = 0;
+    int max_nlong = 0;
+    for (int c = 0; c < nch; ++c) {
+        l0[c] = (int)lrow.size();
+        long long toff = 0;
+        for (int u = c * rows; u < std::min(U, (c + 1) * rows); ++u) {
+            if (Mu[u] > bmm::LOO_SHORT_MAX_M) {
+                lrow.push_back(u - c * rows);
+                lM.push_back(Mu[u]);
+                ltoff.push_back(toff);
+                toff += Mu[u];
+                long_m[c] = std::max(long_m[c], Mu[u]);
+            } else {
+                short_m[c] = std::max(short_m[c], Mu[u]);
+            }
+        }
+        max_tail = std::max(max_tail, toff);
+        max_nlong = std::max(max_nlong, (int)lrow.size() - l0[c]);
+    }
+    l0[nch] = (int)lrow.size();
+    const int nblk = bmm::loo_long_blocks(D);
+    DevBuf dM, dlrow, dlM, dltoff, sel, hist, tail, part, out;
+    TRY(upload(dM, Mu.data(), Mu.size()));
+    if (max_nlong) {
+        TRY(upload(dlrow, lrow.data(), lrow.size()));
+        TRY(upload(dlM, lM.data(), lM.size()));
+        TRY(upload(dltoff, ltoff.data(), ltoff.size()));
+        CU(sel.alloc((size_t)max_nlong * sizeof(bmm::LooSel), false));
+        CU(hist.alloc((size_t)max_nlong * 256 * 4, false));
+        CU(tail.alloc((size_t)max_tail * 8, false));
+        CU(part.alloc((size_t)max_nlong * nblk * 4 * 8, false));
+    }
+    CU(out.alloc((size_t)4 * U * 8, false));
+    double *dE = out.as<double>(), *dL = dE + U, *dK = dL + U, *dN = dK + U;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    CU(cudaEventCreate(&e0));
+    CU(cudaEventCreate(&e1));
+    struct EvPair { cudaEvent_t a, b; ~EvPair() { cudaEventDestroy(a); cudaEventDestroy(b); } } evs{e0, e1};
+    CU(cudaEventRecord(e0, 0));
+    TRY(lm.tables());
+    for (int c = 0; c < nch; ++c) {
+        const int u0 = c * rows, n = std::min(rows, U - u0), nl = l0[c + 1] - l0[c];
+        TRY(lm.produce(u0, n));
+        const double *L = lm.L.as<double>();
+        CU(bmm::launch_loo_short(n, D, short_m[c], L, dM.as<int>() + u0, dE + u0, dL + u0, dK + u0, dN + u0, 0));
+        if (nl)
+            CU(bmm::launch_loo_long(n, D, nl, long_m[c], L, dlrow.as<int>() + l0[c], dlM.as<int>() + l0[c],
+                                    dltoff.as<long long>() + l0[c], sel.as<bmm::LooSel>(), hist.as<unsigned>(),
+                                    tail.as<double>(), part.as<double>(), dE + u0, dL + u0, dK + u0, dN + u0, 0));
+    }
+    CU(cudaEventRecord(e1, 0));
+    CU(cudaEventSynchronize(e1));
+    CU(cudaEventElapsedTime(&g_loo_ms, e0, e1));
+    g_loo_tensor = lm.tensor;
+    TRY(lm.status());
+    std::vector<double> res((size_t)4 * U);
+    CU(cudaMemcpy(res.data(), out.p, res.size() * 8, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < N; ++i) {
+        const int u = rowid[i];
+        if (elpd_loo) elpd_loo[i] = res[u];
+        if (lpd) lpd[i] = res[(size_t)U + u];
+        if (pareto_k) pareto_k[i] = res[(size_t)2 * U + u];
+        if (n_eff) n_eff[i] = res[(size_t)3 * U + u] * (r_eff ? r_eff[i] : 1.0);
+    }
+    return BMM_OK;
+}
+
+int bmm_loo_kernel_ms(float *ms, int32_t *tensor) {
+    if (!ms || !tensor) return fail(BMM_ERR_INVALID, "ms / tensor is NULL");
+    *ms = g_loo_ms;
+    *tensor = g_loo_tensor;
+    return BMM_OK;
+}
+
+int bmm_loglik_matrix(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta,
+                      const double *pi, uint32_t flags, int32_t device, double *out) {
+    TRY(loglik_args(X, N, P, K, S, C, theta, pi, "loglik_matrix"));
+    if (!out) return fail(BMM_ERR_INVALID, "loglik_matrix: out is NULL");
+    if (device < 0 || bmm_device_count() <= device) return fail(BMM_ERR_CUDA, "no CUDA device (this library has no CPU fallback)");
+    const long long D = (long long)C * S;
+    std::vector<uint32_t> bits;
+    int W;
+    TRY(input_rows(X, N, P, flags, bits, W));
+    std::vector<int> rowid, wt;
+    std::vector<uint32_t> rowbits;
+    dedup_rows(bits.data(), N, W, rowid, wt, rowbits);
+    std::vector<uint32_t>().swap(bits);
+    const int U = (int)wt.size();
+    LoglikMat lm;
+    TRY(lm.init(rowbits, U, W, P, K, S, C, theta, pi, flags, device));
+    TRY(lm.tables());
+    std::vector<double> h;
+    for (int u0 = 0; u0 < U; u0 += lm.rows) {
+        const int n = std::min(lm.rows, U - u0);
+        TRY(lm.produce(u0, n));
+        h.resize((size_t)n * D);
+        CU(cudaMemcpy(h.data(), lm.L.p, h.size() * 8, cudaMemcpyDeviceToHost));
+        TRY(lm.status());
+        for (int i = 0; i < N; ++i) {
+            const int u = rowid[i] - u0;
+            if (u < 0 || u >= n) continue;
+            double *o = out + (size_t)D * i;
+            for (long long g = 0; g < D; ++g) o[g] = h[(size_t)g * n + u];
+        }
+    }
     return BMM_OK;
 }
 

@@ -12,6 +12,7 @@
 // leaves the multiplicity-weighted sum of l.  waic_merge_kernel combines slices into chains and chains into the pooled
 // figure in a fixed order (Chan et al.'s variance merge), waic_sum_kernel sums partials in a fixed order: no atomics, so
 // two calls return the same bits.  The tcgen05 kernel (kern_waic_tc.cu) leaves the same partials, one slice per chain.
+// loglik_fp64_kernel stores the same l[g,u] of a chunk of distinct rows instead, the matrix PSIS-LOO reads (kern_loo.cu).
 #include "kernels.h"
 
 namespace bmm {
@@ -67,6 +68,20 @@ __global__ void __launch_bounds__(128) predict_kernel(int M, int P, int W, int K
     logpred[m] = acc > 0.0 ? mx + log(acc) - log((double)S) : -INFINITY;
 }
 
+// l = log sum_k exp(tab[g][k][2P] + sum_d tab[g][k][d or P + d]) of one packed row under draw g
+__device__ __forceinline__ double draw_loglik(const uint32_t *xb, const double *tab, size_t g, int K, int P) {
+    const size_t row = 2 * P + 1;
+    double lmx = -INFINITY, lsum = 0.0;
+    for (int k = 0; k < K; ++k) {
+        const double *t = tab + (g * K + k) * row;
+        double ll = t[2 * P];
+        for (int d = 0; d < P; ++d) ll += ((xb[d >> 5] >> (d & 31)) & 1u) ? t[d] : t[P + d];
+        if (ll > lmx) { lsum = lsum * exp(lmx - ll) + 1.0; lmx = ll; }
+        else if (ll > -INFINITY) lsum += exp(ll - lmx);
+    }
+    return lsum > 0.0 ? lmx + log(lsum) : -INFINITY;
+}
+
 __global__ void __launch_bounds__(128) waic_fp64_kernel(int U, int P, int W, int K, int S, int CQ, int Q, int SL, int ntiles,
                                                         const uint32_t *__restrict__ rowbits, const int *__restrict__ wt,
                                                         const double *__restrict__ tab, double *__restrict__ stat,
@@ -79,20 +94,11 @@ __global__ void __launch_bounds__(128) waic_fp64_kernel(int U, int P, int W, int
     const bool valid = u < U;
     const uint32_t *xb = rowbits + (size_t)(valid ? u : 0) * W;
     const double w = valid ? (double)wt[u] : 0.0;
-    const size_t row = 2 * P + 1;
     double st[WAIC_STAT];
     waic_stat_init(st);
     for (int s = s0; s < s1; ++s) {
         const size_t g = (size_t)c * S + s;
-        double lmx = -INFINITY, lsum = 0.0;
-        for (int k = 0; k < K; ++k) {
-            const double *t = tab + (g * K + k) * row;
-            double ll = t[2 * P];
-            for (int d = 0; d < P; ++d) ll += ((xb[d >> 5] >> (d & 31)) & 1u) ? t[d] : t[P + d];
-            if (ll > lmx) { lsum = lsum * exp(lmx - ll) + 1.0; lmx = ll; }
-            else if (ll > -INFINITY) lsum += exp(ll - lmx);
-        }
-        const double l = lsum > 0.0 ? lmx + log(lsum) : -INFINITY;
+        const double l = draw_loglik(xb, tab, g, K, P);
         waic_push(st, l);
         double v = valid ? w * l : 0.0;
 #pragma unroll
@@ -101,6 +107,23 @@ __global__ void __launch_bounds__(128) waic_fp64_kernel(int U, int P, int W, int
     }
     if (valid)
         for (int e = 0; e < WAIC_STAT; ++e) stat[((size_t)q * U + u) * WAIC_STAT + e] = st[e];
+}
+
+// L[g Uc + u] = l of distinct row u under draw g; one warp per (tile of 32 rows, slice of SL draws), lane = row
+__global__ void __launch_bounds__(128) loglik_fp64_kernel(int Uc, int P, int W, int K, long long D, long long SL, int nslices,
+                                                          int ntiles, const uint32_t *__restrict__ rowbits,
+                                                          const double *__restrict__ tab, double *__restrict__ L) {
+    const int lane = threadIdx.x & 31, tile = blockIdx.x % ntiles;
+    const int q = (blockIdx.x / ntiles) * 4 + (threadIdx.x >> 5);
+    if (q >= nslices) return;
+    const int u = tile * 32 + lane;
+    const bool valid = u < Uc;
+    const uint32_t *xb = rowbits + (size_t)(valid ? u : 0) * W;
+    const long long g1 = min(D, (q + 1) * SL);
+    for (long long g = q * SL; g < g1; ++g) {
+        const double l = draw_loglik(xb, tab, (size_t)g, K, P);
+        if (valid) L[(size_t)g * Uc + u] = l;
+    }
 }
 
 // One thread per distinct row: chain c = merge of its Q slices in order, pooled = merge of the chains in order.
@@ -160,6 +183,19 @@ cudaError_t launch_waic_fp64(int U, int P, int W, int K, int S, int C, int Q, co
     const long long blocks = (long long)ntiles * ((C * Q + 3) / 4);
     if (blocks > 0x7FFFFFFFLL) return cudaErrorInvalidConfiguration;
     waic_fp64_kernel<<<(unsigned)blocks, 128, 0, st>>>(U, P, W, K, S, C * Q, Q, SL, ntiles, rowbits, wt, tab, stat, tpart);
+    g_launches++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_loglik_fp64(int Uc, int P, int W, int K, long long D, const uint32_t *rowbits, const double *tab,
+                               double *L, cudaStream_t st) {
+    const int ntiles = (Uc + 31) / 32;
+    long long q = 32768 / ntiles;                                 // enough warps to fill the GPU several times over
+    q = q < 1 ? 1 : (q > D ? D : q);
+    const long long SL = (D + q - 1) / q, nslices = (D + SL - 1) / SL;
+    const long long blocks = (long long)ntiles * ((nslices + 3) / 4);
+    if (blocks > 0x7FFFFFFFLL) return cudaErrorInvalidConfiguration;
+    loglik_fp64_kernel<<<(unsigned)blocks, 128, 0, st>>>(Uc, P, W, K, D, SL, (int)nslices, ntiles, rowbits, tab, L);
     g_launches++;
     return cudaGetLastError();
 }

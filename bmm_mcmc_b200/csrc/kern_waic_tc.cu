@@ -15,6 +15,10 @@
 // Every wait on an mbarrier is bounded; a time-out sets *status = BMM_ERR_TIMEOUT.  The partials have the layout of the
 // fp64 path (kern_predict.cu) with one slice per chain, and waic_merge_kernel / waic_sum_kernel combine them in a fixed
 // order: the results do not depend on the grid size.
+//
+// With LMAT = true (launch_loglik_tc) the epilogue stores l itself, L[g U + u] over the D draws of one pooled chain (the
+// log-likelihood matrix PSIS-LOO reads, kern_loo.cu), lane = row so a warp's store is 256 contiguous bytes, and keeps no
+// moments.  The WAIC instantiation (LMAT = false) is unchanged.
 #include <cstdlib>
 #include <cuda_fp16.h>
 
@@ -66,7 +70,7 @@ struct WtLayout {
     static constexpr int LAUNCH = TOTAL > 50 * 1024 ? TOTAL : 50 * 1024;
 };
 
-template <int NCH>
+template <int NCH, bool LMAT>
 __global__ void __launch_bounds__(WT_THREADS) waic_tc_kernel(int U, int W, int S, int C, const uint32_t *__restrict__ rowbits,
                                                              const int *__restrict__ wt, const unsigned char *__restrict__ img,
                                                              const float *__restrict__ bias, double *__restrict__ stat,
@@ -170,7 +174,7 @@ __global__ void __launch_bounds__(WT_THREADS) waic_tc_kernel(int U, int W, int S
             }
             fence_async_smem();
             mbar_arrive(a_full);
-            const double w = valid ? (double)wt[u] : 0.0;
+            const double w = (!LMAT && valid) ? (double)wt[u] : 0.0;
             double st[WAIC_STAT];
             waic_stat_init(st);
             int c = 0, s = 0;
@@ -211,6 +215,11 @@ __global__ void __launch_bounds__(WT_THREADS) waic_tc_kernel(int U, int W, int S
                     asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(lg) : "f"(sum));
                     l = ((double)mx + (double)lg) * 0.6931471805599453;
                 }
+                if constexpr (LMAT) {
+                    if (valid) stat[(size_t)g * U + u] = l;
+                    if (++a == WT_NA) { a = 0; ph_a ^= 1u; }
+                    continue;
+                }
                 waic_push(st, l);
                 double v = valid ? w * l : 0.0;
 #pragma unroll
@@ -236,21 +245,21 @@ __global__ void __launch_bounds__(WT_THREADS) waic_tc_kernel(int U, int W, int S
     }
 }
 
-template <int NCH>
+template <int NCH, bool LMAT>
 cudaError_t launch_tc_nch(int U, int W, int S, int C, const uint32_t *rowbits, const int *wt, const unsigned char *img,
                           const float *bias, double *stat, double *tpart, int *status, int sm_count, cudaStream_t st) {
     using L = WtLayout<NCH>;
     static FuncAttrCache attr;
-    if (cudaError_t e = attr.ensure_smem(waic_tc_kernel<NCH>, (int)L::LAUNCH)) return e;
+    if (cudaError_t e = attr.ensure_smem(waic_tc_kernel<NCH, LMAT>, (int)L::LAUNCH)) return e;
     int per_sm = 0;
-    if (cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, waic_tc_kernel<NCH>, WT_THREADS, (size_t)L::LAUNCH))
+    if (cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, waic_tc_kernel<NCH, LMAT>, WT_THREADS, (size_t)L::LAUNCH))
         return e;
     const long long ntiles = ((long long)U + 127) / 128;
     long long ctas = (long long)sm_count * (per_sm < 1 ? 1 : per_sm);
     if (ctas > ntiles) ctas = ntiles;
     if (const char *e = getenv("BMM_GRID_MAX_CTAS")) { const int cap = atoi(e); if (cap > 0 && ctas > cap) ctas = cap; }   // tests: many tiles per CTA
     if (ctas < 1) ctas = 1;
-    waic_tc_kernel<NCH><<<(unsigned)ctas, WT_THREADS, (size_t)L::LAUNCH, st>>>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status);
+    waic_tc_kernel<NCH, LMAT><<<(unsigned)ctas, WT_THREADS, (size_t)L::LAUNCH, st>>>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status);
     g_launches++;
     return cudaGetLastError();
 }
@@ -272,13 +281,26 @@ cudaError_t launch_waic_tc(int U, int P, int W, int K, int S, int C, const uint3
                            int sm_count, cudaStream_t st) {
     (void)K;
     switch (ws_nch(P)) {
-        case 2: return launch_tc_nch<2>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        case 4: return launch_tc_nch<4>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        case 6: return launch_tc_nch<6>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        case 8: return launch_tc_nch<8>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        case 10: return launch_tc_nch<10>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        case 12: return launch_tc_nch<12>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
-        default: return launch_tc_nch<14>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 2: return launch_tc_nch<2, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 4: return launch_tc_nch<4, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 6: return launch_tc_nch<6, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 8: return launch_tc_nch<8, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 10: return launch_tc_nch<10, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        case 12: return launch_tc_nch<12, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+        default: return launch_tc_nch<14, false>(U, W, S, C, rowbits, wt, img, bias, stat, tpart, status, sm_count, st);
+    }
+}
+
+cudaError_t launch_loglik_tc(int Uc, int P, int W, long long D, const uint32_t *rowbits, const unsigned char *img,
+                             const float *bias, double *L, int *status, int sm_count, cudaStream_t st) {
+    switch (ws_nch(P)) {
+        case 2: return launch_tc_nch<2, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        case 4: return launch_tc_nch<4, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        case 6: return launch_tc_nch<6, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        case 8: return launch_tc_nch<8, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        case 10: return launch_tc_nch<10, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        case 12: return launch_tc_nch<12, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
+        default: return launch_tc_nch<14, true>(Uc, W, (int)D, 1, rowbits, nullptr, img, bias, L, nullptr, status, sm_count, st);
     }
 }
 

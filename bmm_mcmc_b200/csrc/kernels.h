@@ -337,6 +337,34 @@ cudaError_t launch_waic_tc(int U, int P, int W, int K, int S, int C, const uint3
                            const unsigned char *img, const float *bias, double *stat, double *tpart, int *status,
                            int sm_count, cudaStream_t st);
 
+// ---- PSIS-LOO and the log-likelihood matrix (kern_predict.cu / kern_waic_tc.cu producers, kern_loo.cu) ----------------
+// L [D][Uc]: l of the Uc distinct rows rowbits [Uc][W] under each of the D pooled draws.  fp64 from launch_predict_tables'
+// tables over the D draws; tcgen05 (waic_tc_supported shapes) from launch_waic_tc_tables' images.
+cudaError_t launch_loglik_fp64(int Uc, int P, int W, int K, long long D, const uint32_t *rowbits, const double *tab,
+                               double *L, cudaStream_t st);
+cudaError_t launch_loglik_tc(int Uc, int P, int W, long long D, const uint32_t *rowbits, const unsigned char *img,
+                             const float *bias, double *L, int *status, int sm_count, cudaStream_t st);
+// Rows whose Pareto tail has at most LOO_SHORT_MAX_M draws take one thread each, longer tails (up to LOO_MAX_TAIL draws,
+// sorted in shared memory) a radix select over several CTAs.
+constexpr int LOO_SHORT_MAX_M = 64;
+constexpr int LOO_MAX_TAIL = 16384;
+// radix-select state of one long row: selected key prefix, rank still to find, keys above the prefix, max / min key,
+// tail draws gathered
+struct LooSel {
+    unsigned long long prefix, kmax, kmin;
+    unsigned rank, gt, tcount, pad;
+};
+int loo_long_blocks(long long D);
+// Outputs per chunk row (elpd, lpd, khat, neff, each [Uc]); Mrow [Uc] = tail length of each row (rows with
+// Mrow > LOO_SHORT_MAX_M are skipped); max_m = the largest Mrow <= LOO_SHORT_MAX_M (sizes shared memory).
+cudaError_t launch_loo_short(int Uc, long long D, int max_m, const double *L, const int *Mrow, double *elpd, double *lpd,
+                             double *khat, double *neff, cudaStream_t st);
+// nlong rows lrow [nlong] of the chunk with tail lengths lM (> LOO_SHORT_MAX_M, <= LOO_MAX_TAIL, max_m the largest) and
+// tail storage tail + ltoff[r]; scratch sel [nlong], hist [nlong][256], part [nlong][loo_long_blocks(D)][4]
+cudaError_t launch_loo_long(int Uc, long long D, int nlong, int max_m, const double *L, const int *lrow, const int *lM,
+                            const long long *ltoff, LooSel *sel, unsigned *hist, double *tail, double *part, double *elpd,
+                            double *lpd, double *khat, double *neff, cudaStream_t st);
+
 // ---- history layout conversion (kern_finalize.cu) --------------------------------------------
 // zhist [c][nsamples][N] uint8 -> R layout [c][S x N cm]; optional relabelling through perm_out.
 // elem_bytes = 4 (int32) or 1 (uint8, BMM_FLAG_COMPACT_Z).

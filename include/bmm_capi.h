@@ -51,8 +51,8 @@ extern "C" {
                                         uint32 [N][ceil(P/32)], bit d%32 of word d/32 = x_id (grid
                                         path only; 8 B per row at P = 64 instead of 256 B)         */
 #define BMM_FLAG_NO_TENSOR 32u        /* grid path, BMM_FP32: use the CUDA-core float kernel instead of
-                                        the tcgen05 contraction (A/B testing); bmm_waic: the fp64
-                                        kernel                                                     */
+                                        the tcgen05 contraction (A/B testing); bmm_waic, bmm_loo,
+                                        bmm_loglik_matrix: the fp64 kernel                         */
 #define BMM_FLAG_STEPHENS_FIXED 64u   /* correctness-fixed relabelling (NOT the reference, SURVEY 8f-3): the batch
                                       * initialisation and the online Q update re-order columns with the
                                       * inverse of index_max(solution.col(.)) -- what the no-op
@@ -200,6 +200,27 @@ int bmm_waic(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t 
              double *chain_p_waic);
 /* Device time in ms of the last bmm_waic's kernels on this thread, and 1 if it took the tcgen05 kernel.               */
 int bmm_waic_kernel_ms(float *ms, int32_t *tensor);
+/* PSIS-LOO (Vehtari, Gelman & Gabry 2017; as R's loo::loo, without mcse_elpd_loo) of a fitted gibbs_full /
+ * gibbs_stickbreaking model (no reference counterpart).  X, theta, pi, flags and device as bmm_waic; r_eff: NULL (1) or
+ * N relative efficiencies > 0, which set each observation's Pareto tail length M = min(ceil(0.2 D), ceil(3 sqrt(D / r_eff)))
+ * (D = C S; M <= 16384, so D <= 29826161 at r_eff = 1).  With l[g, i] the log-likelihood of observation i under pooled
+ * draw g and w~ the Pareto-smoothed, truncated, normalised log weights of r = -l:
+ *   elpd_loo [N]   log sum_g exp(w~_g + l[g, i])
+ *   lpd [N]        log 1/D sum_g exp l[g, i] (WAIC's lppd)
+ *   pareto_k [N]   the tail's generalized Pareto shape (inf when M < 5 or the tail is flat)
+ *   n_eff [N]      r_eff_i / sum_g exp(2 w~_g)
+ * Any output may be NULL.  Computed on the device in a fixed order (two calls return the same bits).  theta exactly 0 or 1
+ * can give l = -inf; then elpd_loo and n_eff are nan and pareto_k inf, as the float64 definition gives.              */
+int bmm_loo(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta, const double *pi,
+            const double *r_eff, uint32_t flags, int32_t device, double *elpd_loo, double *lpd, double *pareto_k,
+            double *n_eff);
+/* Device time in ms of the last bmm_loo's kernels on this thread, and 1 if its log-likelihood matrix came from the
+ * tcgen05 kernel.                                                                                                       */
+int bmm_loo_kernel_ms(float *ms, int32_t *tensor);
+/* The log-likelihood matrix out [(C S) x N] column-major, out[g + C S i] = l[g, i] over the chain-major pooled draws
+ * g = c S + s: the draws x observations matrix loo::loo() takes.  Inputs as bmm_waic.                                 */
+int bmm_loglik_matrix(const void *X, int32_t N, int32_t P, int32_t K, int32_t S, int32_t C, const double *theta,
+                      const double *pi, uint32_t flags, int32_t device, double *out);
 
 /* Diagnostic (no reference counterpart): %globaltimer stamps in ns of the last two sweeps of the tensor grid path.
  * out[8 * (j & 1) + s], z-sweep kernel CTA 0: s = 0 entry, 1 pipeline start, 2 first tile drawn, 3 last tile drawn,

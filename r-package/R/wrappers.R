@@ -90,3 +90,42 @@ waic_gibbs <- function(obj, data) {
     colnames(r$pointwise) <- c("elpd_waic", "p_waic", "waic")
     r
 }
+
+#' PSIS-LOO of a fitted model
+#'
+#' Not in the reference: Pareto-smoothed importance-sampling leave-one-out cross-validation (Vehtari, Gelman & Gabry
+#' 2017) of an uncollapsed fit, computed on the GPU, in the layout of \code{loo::loo} (lower \code{looic} is better).
+#' Observations with \code{pareto_k} above 0.7 have an unreliable estimate.  \code{mcse_elpd_loo} is not computed:
+#' current \code{loo} estimates it from random gamma draws, which cannot be reproduced.
+#'
+#' @param obj The list returned by \code{gibbs_full} or \code{gibbs_stickbreaking}.
+#' @param data The N x P 0/1 matrix the model was fitted to.
+#' @param r_eff Relative efficiency of the draws, one value or one per observation (e.g. from \code{loo::relative_eff}).
+#' @return A list with \code{estimates} (rows elpd_loo, p_loo, looic; columns Estimate, SE), \code{pointwise} (N x 4:
+#'   elpd_loo, p_loo, looic, influence_pareto_k) and \code{diagnostics} (\code{pareto_k}, \code{n_eff}).
+#' @export
+loo_gibbs <- function(obj, data, r_eff = 1) {
+    if (is.null(obj$pi)) stop("loo_gibbs needs the pi history of gibbs_full / gibbs_stickbreaking")
+    data <- as.matrix(data)
+    storage.mode(data) <- "integer"
+    r <- loo_cpp(data, obj$theta, obj$pi, as.numeric(r_eff))
+    dimnames(r$estimates) <- list(c("elpd_loo", "p_loo", "looic"), c("Estimate", "SE"))
+    colnames(r$pointwise) <- c("elpd_loo", "p_loo", "looic", "influence_pareto_k")
+    r
+}
+
+#' Log-likelihood matrix of a fitted model
+#'
+#' Not in the reference: the S x N matrix of log p(x_i | draw s) over the kept draws, computed on the GPU, as
+#' \code{loo::loo()} and \code{loo::waic()} take it.
+#'
+#' @param obj The list returned by \code{gibbs_full} or \code{gibbs_stickbreaking}.
+#' @param data The N x P 0/1 matrix the model was fitted to.
+#' @return An S x N numeric matrix.
+#' @export
+log_lik_gibbs <- function(obj, data) {
+    if (is.null(obj$pi)) stop("log_lik_gibbs needs the pi history of gibbs_full / gibbs_stickbreaking")
+    data <- as.matrix(data)
+    storage.mode(data) <- "integer"
+    log_lik_cpp(data, obj$theta, obj$pi)
+}

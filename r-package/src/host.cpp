@@ -181,6 +181,59 @@ List waic_cpp(IntegerMatrix data, NumericVector theta, NumericMatrix pi) {
     return List::create(Named("estimates") = estimates, Named("pointwise") = pointwise, Named("loglik") = loglik);
 }
 
+// PSIS-LOO of a fitted model (no reference counterpart; the layout of loo::loo without mcse_elpd_loo, which current loo
+// estimates by random gamma draws that cannot be reproduced): estimates 3 x 2 (rows elpd_loo, p_loo, looic; columns
+// Estimate, SE = sqrt(N var(pointwise))), pointwise N x 4 (elpd_loo, p_loo, looic, influence_pareto_k), diagnostics =
+// list(pareto_k, n_eff).  r_eff: one value, or one per observation (> 0).  theta, pi and data as waic_cpp.
+// [[Rcpp::export]]
+List loo_cpp(IntegerMatrix data, NumericVector theta, NumericMatrix pi, NumericVector r_eff) {
+    IntegerVector dim = theta.attr("dim");
+    if (dim.size() != 3) stop("theta must be a K x P x S array");
+    const int K = dim[0], P = dim[1], S = dim[2], N = data.nrow();
+    if (data.ncol() != P || pi.nrow() != S || pi.ncol() != K) stop("data / theta / pi dimensions do not match");
+    if (S < 2) stop("loo needs at least 2 draws");
+    if (r_eff.size() != 1 && r_eff.size() != N) stop("r_eff must have length 1 or one value per observation");
+    NumericVector re(N), elpd(N), lpd(N), k(N), n_eff(N);
+    for (int i = 0; i < N; ++i) {
+        re[i] = r_eff[r_eff.size() == 1 ? 0 : i];
+        if (!(re[i] > 0.0) || !std::isfinite(re[i])) stop("r_eff must be finite and > 0");
+    }
+    if (bmm_loo(data.begin(), N, P, K, S, 1, theta.begin(), pi.begin(), re.begin(), 0u, 0, elpd.begin(), lpd.begin(),
+                k.begin(), n_eff.begin()) != BMM_OK)
+        stop(bmm_last_error());
+    NumericMatrix pointwise(N, 4), estimates(3, 2);
+    for (int i = 0; i < N; ++i) {
+        pointwise(i, 0) = elpd[i];
+        pointwise(i, 1) = lpd[i] - elpd[i];
+        pointwise(i, 2) = -2.0 * elpd[i];
+        pointwise(i, 3) = k[i];
+    }
+    for (int j = 0; j < 3; ++j) {
+        double sum = 0.0, ss = 0.0;
+        for (int i = 0; i < N; ++i) sum += pointwise(i, j);
+        const double mean = sum / N;
+        for (int i = 0; i < N; ++i) ss += (pointwise(i, j) - mean) * (pointwise(i, j) - mean);
+        estimates(j, 0) = sum;
+        estimates(j, 1) = N > 1 ? std::sqrt(N * (ss / (N - 1))) : NAN;
+    }
+    return List::create(Named("estimates") = estimates, Named("pointwise") = pointwise,
+                        Named("diagnostics") = List::create(Named("pareto_k") = k, Named("n_eff") = n_eff));
+}
+
+// The S x N log-likelihood matrix l[s, i] = log p(x_i | draw s) that loo::loo() takes.  theta, pi and data as waic_cpp.
+// [[Rcpp::export]]
+NumericMatrix log_lik_cpp(IntegerMatrix data, NumericVector theta, NumericMatrix pi) {
+    IntegerVector dim = theta.attr("dim");
+    if (dim.size() != 3) stop("theta must be a K x P x S array");
+    const int K = dim[0], P = dim[1], S = dim[2], N = data.nrow();
+    if (data.ncol() != P || pi.nrow() != S || pi.ncol() != K) stop("data / theta / pi dimensions do not match");
+    if (S < 2) stop("log_lik needs at least 2 draws");
+    NumericMatrix out(S, N);
+    if (bmm_loglik_matrix(data.begin(), N, P, K, S, 1, theta.begin(), pi.begin(), 0u, 0, out.begin()) != BMM_OK)
+        stop(bmm_last_error());
+    return out;
+}
+
 // Posterior predictive distribution (no reference counterpart; the reference's TODO:6 lists it).  theta: K x P x S array
 // and pi: S x K matrix as gibbs_full / gibbs_stickbreaking return them; newdata: M x P 0/1 integer matrix.
 // [[Rcpp::export]]
