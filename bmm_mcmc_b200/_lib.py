@@ -54,7 +54,7 @@ class Out(C.Structure):
 
 EXPORTS = [
     "bmm_gibbs_full", "bmm_gibbs_stickbreaking", "bmm_gibbs_collapsed", "bmm_gibbs_dp", "bmm_stephens_batch",
-    "bmm_stephens_online", "bmm_stephens_batch_ex", "bmm_stephens_online_ex", "bmm_assign", "bmm_assign_warp", "bmm_grid_cost", "bmm_rdirichlet", "bmm_predictive", "bmm_waic", "bmm_waic_kernel_ms", "bmm_loo", "bmm_loo_kernel_ms", "bmm_loglik_matrix", "bmm_debug_ws_trace", "bmm_debug_ws_cta", "bmm_full_condprob", "bmm_plan_create", "bmm_plan_run",
+    "bmm_stephens_online", "bmm_stephens_batch_ex", "bmm_stephens_online_ex", "bmm_assign", "bmm_assign_warp", "bmm_grid_cost", "bmm_rdirichlet", "bmm_predictive", "bmm_waic", "bmm_waic_kernel_ms", "bmm_loo", "bmm_loo_kernel_ms", "bmm_loglik_matrix", "bmm_debug_ws_trace", "bmm_debug_ws_cta", "bmm_debug_chain_kernel", "bmm_debug_chain_phases", "bmm_full_condprob", "bmm_plan_create", "bmm_plan_run",
     "bmm_plan_sync", "bmm_plan_elapsed_ms", "bmm_plan_fetch", "bmm_plan_destroy", "bmm_dist_unique_id",
     "bmm_dist_init", "bmm_dist_finalize", "bmm_dist_p2p_local", "bmm_dist_p2p_attach", "bmm_dist_p2p_detach", "bmm_plan_kernel_ms", "bmm_host_alloc", "bmm_host_free", "bmm_release_cache", "bmm_last_error", "bmm_device_count", "bmm_launch_count", "bmm_fetch_bytes", "bmm_version",
 ]
@@ -92,6 +92,7 @@ def lib():
                                     C.POINTER(C.c_double)]
         L.bmm_waic.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _dbl_p, _dbl_p,
                                C.c_uint32, C.c_int32, _dbl_p, _dbl_p, _dbl_p, _dbl_p, _dbl_p]
+        L.bmm_debug_chain_phases.argtypes = [C.POINTER(C.c_uint64), C.c_int64]
         L.bmm_waic_kernel_ms.argtypes = [C.POINTER(C.c_float), C.POINTER(C.c_int32)]
         L.bmm_loo.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _dbl_p, _dbl_p, _dbl_p,
                               C.c_uint32, C.c_int32, _dbl_p, _dbl_p, _dbl_p, _dbl_p]

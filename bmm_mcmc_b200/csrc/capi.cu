@@ -854,11 +854,21 @@ int full_threads(int n_chains) {
     return n_chains >= 512 ? 64 : 128;
 }
 
+// Kernel of the last chain-per-block launch of the uncollapsed samplers (bmm_debug_chain_kernel): 1 full_chain_kernel,
+// 2 chain_sweep_kernel.
+int g_chain_kernel = 0;
+
 int run_segment(bmm_plan *pl, int j0, int j1) {
     if (j1 <= j0) return BMM_OK;
     if (pl->sampler == BMM_SAMPLER_FULL || pl->sampler == BMM_SAMPLER_STICKBREAKING) {
         pl->fp.j_begin = j0; pl->fp.j_end = j1;
-        CU(bmm::launch_full(pl->fp, pl->C, full_threads(pl->C), pl->stream));
+        const int threads = full_threads(pl->C);
+        // the specialised sweep kernel where it applies; BMM_CHAIN_KERNEL=generic keeps full_chain_kernel (tests, A/B)
+        const char *force = getenv("BMM_CHAIN_KERNEL");
+        const bool sweep = !(force && !strcmp(force, "generic")) && bmm::chain_sweep_supported(pl->fp, threads);
+        g_chain_kernel = sweep ? 2 : 1;
+        if (sweep) CU(bmm::launch_chain_sweep(pl->fp, pl->C, threads, pl->stream));
+        else CU(bmm::launch_full(pl->fp, pl->C, threads, pl->stream));
     } else {
         pl->cp.j_begin = j0; pl->cp.j_end = j1;
         CU(bmm::launch_collapsed(pl->cp, pl->C, pl->stream));
@@ -1463,6 +1473,17 @@ int bmm_debug_ws_trace(uint64_t out[32]) {
     CU(bmm::ws_trace_read(t));
     CU(bmm::upd_trace_read(t + 16));
     for (int i = 0; i < 32; ++i) out[i] = t[i];
+    return BMM_OK;
+}
+
+int bmm_debug_chain_kernel(void) { return g_chain_kernel; }
+
+int bmm_debug_chain_phases(uint64_t *out, int64_t n) {
+    if (!out || n < 0) return fail(BMM_ERR_INVALID, "out is NULL or n < 0");
+    CU(cudaDeviceSynchronize());
+    bool supported = false;
+    CU(bmm::chain_phase_read((unsigned long long *)out, (size_t)n, &supported));
+    if (!supported) return fail(BMM_ERR_UNSUPPORTED, "built without BMM_CHAIN_PHASE_CLOCKS");
     return BMM_OK;
 }
 

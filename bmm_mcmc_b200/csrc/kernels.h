@@ -85,6 +85,13 @@ struct FullParams {
 constexpr int COST_SMEM_MAX = 64 * 64;
 size_t full_smem_bytes(const FullParams &p, int threads);
 cudaError_t launch_full(const FullParams &p, int n_chains, int threads, cudaStream_t st);
+// chain_sweep_kernel: the same chain, bit for bit, specialised to Philox mode with the (row, label) histogram and no
+// probes, which is what chain_sweep_supported checks; everything else runs full_chain_kernel
+bool chain_sweep_supported(const FullParams &p, int threads);
+cudaError_t launch_chain_sweep(const FullParams &p, int n_chains, int threads, cudaStream_t st);
+// per-phase cycle totals [chain][warp < 4][9] of builds with -DBMM_CHAIN_PHASE_CLOCKS (read and cleared);
+// *supported = false in the default build
+cudaError_t chain_phase_read(unsigned long long *out, size_t n, bool *supported);
 
 // ---- collapsed finite-K and DP samplers, one chain per warp-sized block (kern_collapsed.cu) ---
 struct CollapsedParams {

@@ -229,6 +229,15 @@ int bmm_loglik_matrix(const void *X, int32_t N, int32_t P, int32_t K, int32_t S,
 int bmm_debug_ws_trace(uint64_t out[32]);
 /* ... and per CTA b of the last launch: out[2b] = (entry ns << 10) | SM id, out[2b + 1] = counts-flushed ns.      */
 int bmm_debug_ws_cta(uint64_t out[320]);
+/* Kernel of the last chain-per-block launch of gibbs_full / gibbs_stickbreaking: 0 none yet, 1 full_chain_kernel (the
+ * generic one), 2 chain_sweep_kernel (Philox mode with the row histogram and no probes; BMM_CHAIN_KERNEL=generic
+ * forces 1).                                                                                                         */
+int bmm_debug_chain_kernel(void);
+/* Per-phase cycle totals of the chain kernels, out[(chain * 4 + warp) * 9 + phase] for chains < 4096, phases A log
+ * tables, B row table, C allocations, D histogram fold, E relabelling, F parameter draws, history write, the wait
+ * after E / F, then the number of sweeps; the totals are cleared by the read.  Only builds with -DBMM_CHAIN_PHASE_CLOCKS (of kern_full.cu)
+ * record them; the default build returns BMM_ERR_UNSUPPORTED.                                                         */
+int bmm_debug_chain_phases(uint64_t *out, int64_t n);
 
 /* ---- probes --------------------------------------------------------------------------------- */
 /* One uncollapsed z-sweep at a given state (full_gibbs.cpp:87-133): log-likelihood and
